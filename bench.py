@@ -5,6 +5,7 @@ top-level line, and the other configurations of BASELINE.json under `workloads` 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one process per GPU under torchrun)
     python bench.py --impl reference --steps K --warmup W    # the reference's own CPU implementation on the host cores
     python bench.py --workload c3|c4|c5 ...                  # one workload as the top-level line (development)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one pass of the hot path over one batch of synthetic input per GPU:
   C2  64 submaps x 4096 points through PointNetVlad(featnet=lpdnet).eval()             batch-sharded, no collective ("weak")
@@ -248,6 +249,16 @@ class Ctx:
         self.flush_buf = torch.empty(256 << 20, dtype=torch.uint8, device=self.device)   # > 126 MB L2
         self.peaks = load_peaks()
         self.steps, self.warmup = args.steps, max(args.warmup, 3)
+        self.outputs = {}             # --dump-outputs: name -> host array of the last timed step
+
+    def keep(self, name, a):
+        """record an output of the last timed step for --dump-outputs (rank 0): floats keep their width, integers (indices,
+        counts) become float64, which holds them exactly"""
+        if not self.args.dump_outputs or self.rank != 0:
+            return
+        import numpy as np
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        self.outputs[name] = a.astype(np.float32 if a.dtype in (np.float16, np.float32) else np.float64)
 
     def pin_cores(self):
         """give every local rank its own slice of the allowed cores (round 1: all 8 ranks shared cores 0-31 of NUMA node 0 and
@@ -371,6 +382,27 @@ class GraphStep:
         self.x.copy_(x, non_blocking=True)
         self.graph.replay()
         return self.y
+
+
+def strided_sample(t, n: int = 4096):
+    """at most n elements of t, evenly strided from its first: the same positions for every build and run"""
+    flat = t.detach().reshape(-1)
+    return flat[::max(1, flat.numel() // n)][:n]
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def write_outputs(out_dir: str, outputs: dict):
+    """--dump-outputs: one DIR/<name>.npy per output of the last timed step"""
+    import numpy as np
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT}-byte limit")
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in outputs.items():
+        np.save(d / f"{name}.npy", a)
 
 
 def reference_modules():
@@ -546,9 +578,10 @@ def bench_embed(ctx, tag: str):
     host = [synth.clouds(B, N, seed=1234 + 97 * ctx.rank + i) for i in range(n_rot)]
     dev_in = [h.to(ctx.device) for h in host]
     step_graph = GraphStep(ctx, model, dev_in[0])
+    state = {}
 
     def step(i):
-        return step_graph(dev_in[i % n_rot])
+        state["out"] = step_graph(dev_in[i % n_rot])
 
     def step_eager(i):
         with torch.no_grad():
@@ -558,6 +591,7 @@ def bench_embed(ctx, tag: str):
         step(i)
     with ClockSampler(ctx.local) as clk:
         t_ms, per_rank, per_step = ctx.timed_steps(step)
+    ctx.keep(f"{tag}_descriptors", state["out"])                     # the graph's output buffer: copy before the next replay
     value = ctx.world * B * ctx.steps / (t_ms * 1e-3)
     launches = step_graph.launches * ctx.steps
     ranks = ctx.rank_report(per_step, clk.result)
@@ -662,6 +696,13 @@ def bench_train(ctx):
     with ClockSampler(ctx.local) as clk:
         t_ms, per_rank, per_step = ctx.timed_steps(step)
     launches = ops.launch_count()
+    if args.dump_outputs:
+        # the caller gets the loss, and the parameters and .grad updated in place (17.6 M values each: a fixed strided sample
+        # of at most 4096 elements per parameter tensor, in model.parameters() order)
+        params = list(model.parameters())
+        ctx.keep("c3_loss", state["loss"].reshape(1))
+        ctx.keep("c3_param_sample", torch.cat([strided_sample(p) for p in params]))
+        ctx.keep("c3_grad_sample", torch.cat([strided_sample(p.grad if p.grad is not None else torch.zeros_like(p)) for p in params]))
     value = ctx.world * TRAIN_CLOUDS * ctx.steps / (t_ms * 1e-3)
     last_loss = float(state["loss"])
     ranks = ctx.rank_report(per_step, clk.result)
@@ -753,6 +794,15 @@ def bench_retrieval(ctx):
     with ClockSampler(ctx.local) as clk:
         t_ms, per_rank, _ = ctx.timed_steps(step)
     launches = ops.launch_count()
+    # the ordered run pairs m != n the evaluation reports ([n][m] tables: the diagonal evaluates no query, its rates are 0 / 0);
+    # sim is NaN where the top-1 is not a true neighbour: kept as 0 there, next to the 0 / 1 hit mask
+    off = ~np.eye(R, dtype=bool)
+    r = state["res"]
+    for name in ("recall", "one_pct", "n_eval"):
+        ctx.keep(f"c4_{name}", r[name][off])
+    hit = ~np.isnan(r["sim"])
+    ctx.keep("c4_sim", np.where(hit, r["sim"], 0.0))
+    ctx.keep("c4_sim_hit", hit)
     value = searches * ctx.steps / (t_ms * 1e-3)                      # fixed total work: strong scaling
 
     # ---- end to end: pinned host descriptors -> H2D -> search + counting -> recall tables on the host ----
@@ -782,6 +832,8 @@ def bench_retrieval(ctx):
     for i in range(3):
         big(i)
     tb_ms, _, _ = ctx.timed_steps(big)
+    ctx.keep("c4_big_idx", state["big"][0])
+    ctx.keep("c4_big_dist", state["big"][1])
     big_qps = q_all.shape[0] * ctx.steps / (tb_ms * 1e-3)
     selfcheck = None
     if ctx.world > 1:
@@ -892,6 +944,8 @@ def run_ours(args):
         line["host"] = {"cores_per_rank": len(ctx.cores), "cpu_count": os.cpu_count()}
         if len(which) > 1:
             line["workloads"] = {w: results[w] for w in which[1:]}
+        if args.dump_outputs:
+            write_outputs(args.dump_outputs, ctx.outputs)
         emit(line)
     if ctx.world > 1:
         ctx.dist.barrier()
@@ -981,7 +1035,13 @@ def main():
                     help="all (default): C2 as the top-level line (the configuration BASELINE.json's metric is quoted on) with C3, C4, C5 "
                          "under `workloads`; or one workload as the top-level line")
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the host-CPU reference samples (development)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of each workload computed as DIR/<name>.npy "
+                         "(float32 / float64, rank 0), so that two builds can be compared output for output: the inputs are "
+                         "seeded and identical for the same arguments")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the CUDA path (--impl ours)")
     quiet_stdout()
     if args.impl == "reference":
         run_reference(args)
