@@ -39,6 +39,29 @@ inline int cuda_fail(cudaError_t e, const char* what, const char* file, int line
         }                                                                           \
     } while (0)
 
+// the tensor-core kernels are built for sm_100a only: LPD_EUNSUPPORTED on any other device
+inline int require_sm100() {
+    int dev = 0, major = 0;
+    LPD_CUDA_CHECK(cudaGetDevice(&dev));
+    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
+    return major == 10 ? LPD_OK : LPD_EUNSUPPORTED;
+}
+
+// SMs of the current device (a persistent kernel launches at most one CTA per SM)
+inline int sm_count(int* sms) {
+    int dev = 0;
+    LPD_CUDA_CHECK(cudaGetDevice(&dev));
+    LPD_CUDA_CHECK(cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, dev));
+    return LPD_OK;
+}
+
+// the activations a fused epilogue applies as act(v) = max(v, v * neg_slope)
+inline bool act_is_slope(int act, float slope) {
+    return act == LPD_ACT_NONE || act == LPD_ACT_RELU || (act == LPD_ACT_LEAKY && slope >= 0.f && slope <= 1.f);
+}
+// neg_slope: 1 -> identity, 0 -> ReLU, 0 < s < 1 -> LeakyReLU(s)
+inline float act_neg_slope(int act, float slope) { return act == LPD_ACT_NONE ? 1.f : (act == LPD_ACT_RELU ? 0.f : slope); }
+
 inline cudaStream_t as_stream(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
 inline int ceil_div(int a, int b) { return (a + b - 1) / b; }

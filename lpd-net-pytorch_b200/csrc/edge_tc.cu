@@ -268,9 +268,9 @@ template <int C1>
 static int dg_tc_launch(const CUtensorMap& tw, DgTcParams P, cudaStream_t st) {
     constexpr size_t smem = 3 * (size_t)(C1 / 32) * DG_ROWS * 128 + 256;
     LPD_CUDA_CHECK(allow_smem(edgeconv_dg_tc_kernel<C1>, smem));
-    int dev = 0, sms = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    const int rc = sm_count(&sms);
+    if (rc != LPD_OK) return rc;
     const int grid = (int)(P.num_tiles < sms ? P.num_tiles : sms);
     edgeconv_dg_tc_kernel<C1><<<grid, DG_THREADS, smem, st>>>(tw, P);
     LPD_LAUNCH_CHECK();
@@ -297,23 +297,20 @@ extern "C" int lpd_edgeconv_dg_tf32(const float* p, int ldp, const float* q, int
     LPD_REQUIRE(ldp >= C1 && ldq >= C1 && ld2 >= C2 && (!x1 || ld1 >= C1));
     LPD_REQUIRE((long long)N * ldp < (1ll << 31));          // cloud-local row offsets are 32-bit
     LPD_REQUIRE(((uintptr_t)p & 15) == 0 && ((uintptr_t)q & 15) == 0 && ((uintptr_t)x1 & 15) == 0 && ((uintptr_t)w2 & 15) == 0);
-    LPD_REQUIRE(act == LPD_ACT_NONE || act == LPD_ACT_RELU || (act == LPD_ACT_LEAKY && slope >= 0.f && slope <= 1.f));
-    int dev = 0, major = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
-    if (major != 10) return LPD_EUNSUPPORTED;
+    LPD_REQUIRE(act_is_slope(act, slope));
+    int rc = require_sm100();
+    if (rc != LPD_OK) return rc;
     if (!s1)    // k = 20, 128 channels, first-layer BatchNorm already applied by the projection GEMM (edge_tc20.cu)
-        return tc::dg20_tc_run(p, ldp, q, ldq, idx, B, N, w2, s2, t2, act == LPD_ACT_NONE ? 1.f : (act == LPD_ACT_RELU ? 0.f : slope),
-                               x1, ld1, x2, ld2, as_stream(stream));
+        return tc::dg20_tc_run(p, ldp, q, ldq, idx, B, N, w2, s2, t2, act_neg_slope(act, slope), x1, ld1, x2, ld2, as_stream(stream));
     tc::DgTcParams P;
     P.p = p; P.q = q; P.idx = idx; P.s1 = s1; P.t1 = t1; P.s2 = s2; P.t2 = t2; P.x1 = x1; P.x2 = x2;
     P.ldp = ldp; P.ldq = ldq; P.ld1 = ld1; P.ld2 = ld2; P.total_pts = (long long)B * N; P.N = N; P.k = k; P.C2 = C2;
-    P.neg_slope = act == LPD_ACT_NONE ? 1.f : (act == LPD_ACT_RELU ? 0.f : slope);
+    P.neg_slope = act_neg_slope(act, slope);
     P.pts_per_tile = tc::DG_ROWS / k;
     P.n_mma = (P.pts_per_tile * k + 15) / 16 * 16;
     P.num_tiles = (P.total_pts + P.pts_per_tile - 1) / P.pts_per_tile;
-    CUtensorMap tw;
-    int rc = tc::make_tmap(&tw, w2, C2, C1, C1, tc::DG_ROWS);   // rows beyond C2 are zero-filled by TMA
+    CUtensorMap tw;   // rows beyond C2 are zero-filled by TMA
+    rc = tc::make_tmap(&tw, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, w2, C2, C1, C1, tc::DG_ROWS, 32);
     if (rc != LPD_OK) return rc;
     cudaStream_t st = as_stream(stream);
     if (C1 == 128) return tc::dg_tc_launch<128>(tw, P, st);

@@ -507,13 +507,13 @@ int dg20_tc_run(const float* p, int ldp, const float* q, int ldq, const int32_t*
     P.neg_slope = neg_slope;
     P.num_tiles = (P.total_pts + D20_PTS - 1) / D20_PTS;
     CUtensorMap tw;
-    int rc = make_tmap(&tw, w2, D20_C, D20_C, D20_C, 128);
+    int rc = make_tmap(&tw, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, w2, D20_C, D20_C, D20_C, 128, 32);
     if (rc != LPD_OK) return rc;
     constexpr size_t smem = 3 * (size_t)D20_OP_BYTES + 256;
     LPD_CUDA_CHECK(allow_smem(edgeconv_dg20_tc_kernel, smem));
-    int dev = 0, sms = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    rc = sm_count(&sms);
+    if (rc != LPD_OK) return rc;
     const int grid = (int)(P.num_tiles < sms ? P.num_tiles : sms);
     edgeconv_dg20_tc_kernel<<<grid, D20_THREADS, smem, st>>>(tw, P);
     LPD_LAUNCH_CHECK();
@@ -532,32 +532,22 @@ static int edgeconv_dgk_f16(const void* p, int ldp, const void* q, int ldq, cons
     LPD_REQUIRE(ldp >= 128 && ldq >= 128 && ld2 >= 128 && (!x1 || ld1 >= 128));
     LPD_REQUIRE((long long)N * ldp < (1ll << 31));
     LPD_REQUIRE(((uintptr_t)p & 15) == 0 && ((uintptr_t)q & 15) == 0 && ((uintptr_t)x1 & 15) == 0 && ((uintptr_t)x2 & 3) == 0 && ((uintptr_t)w2 & 15) == 0);
-    LPD_REQUIRE(act == LPD_ACT_NONE || act == LPD_ACT_RELU || (act == LPD_ACT_LEAKY && slope >= 0.f && slope <= 1.f));
-    int dev = 0, major = 0, sms = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    if (major != 10) return LPD_EUNSUPPORTED;
+    LPD_REQUIRE(act_is_slope(act, slope));
+    int rc = require_sm100();
+    if (rc != LPD_OK) return rc;
+    int sms = 0;
+    rc = sm_count(&sms);
+    if (rc != LPD_OK) return rc;
     tc::Dg20hParams P;
     P.p = reinterpret_cast<const __half*>(p); P.q = reinterpret_cast<const __half*>(q); P.idx = idx; P.s2 = s2; P.t2 = t2;
     P.x1 = reinterpret_cast<__half*>(x1); P.x2 = reinterpret_cast<__half*>(x2);
     P.ldp = ldp; P.ldq = ldq; P.ld1 = ld1; P.ld2 = ld2; P.total_pts = (long long)B * N; P.N = N;
-    P.neg_slope = act == LPD_ACT_NONE ? 1.f : (act == LPD_ACT_RELU ? 0.f : slope);
+    P.neg_slope = act_neg_slope(act, slope);
     const int pts = K == 32 ? tc::DgH<32>::PTS : tc::DgH<20>::PTS;
     P.num_tiles = (P.total_pts + pts - 1) / pts;
-    // W2 fp16 [128][128]: boxes of 64 halves x 128 rows, 128B swizzle
-    tc::EncodeTiledFn enc = tc::get_encode();
-    if (!enc) return LPD_ECUDA;
-    CUtensorMap tw;
-    cuuint64_t dims[2] = {128u, 128u};
-    cuuint64_t strides[1] = {256u};
-    cuuint32_t box[2] = {64u, 128u};
-    cuuint32_t estr[2] = {1, 1};
-    if (enc(&tw, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(w2), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-            CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS) {
-        snprintf(g_last_error, sizeof(g_last_error), "cuTensorMapEncodeTiled (fp16 W2) failed");
-        return LPD_ECUDA;
-    }
+    CUtensorMap tw;   // W2 fp16 [128][128]: boxes of 128 rows x 64 halves
+    rc = tc::make_tmap(&tw, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, w2, 128, 128, 128, 128, 64);
+    if (rc != LPD_OK) return rc;
     constexpr size_t smem = 3 * (size_t)tc::D20H_OP_BYTES + 256;
     const int grid = (int)(P.num_tiles < sms ? P.num_tiles : sms);
     if (K == 32) {

@@ -21,7 +21,6 @@
 // bits, vs the 10-bit TRUNCATION kind::tf32 applies to fp32 operands), twice the tensor rate and half the operand bytes.
 #include "tc_common.cuh"
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 namespace lpd {
 namespace tc {
@@ -33,16 +32,16 @@ constexpr int EPI_WARPS = 8;
 constexpr int THREADS = 64 + 32 * EPI_WARPS;
 
 struct Params {
-    float* C; int ldc; int M, N, K;
-    const float* scale; const float* shift;
-    float neg_slope;   // act(v) = max(v, v * neg_slope): 1 -> identity, 0 -> ReLU, 0 < s < 1 -> LeakyReLU(s)
-    int tiles_m, tiles_n;
-    int batch; long long strideC;   // TN: slice z contracts rows [z*K, (z+1)*K) of both operands into C + z*strideC
-    int bM, bN;                     // !TN, batch > 1: slice z multiplies rows [z*bM, ..) of A with rows [z*bN, ..) of B into C rows z*bM ..
-    int accumulate;                 // !TN: C += result (the epilogue reads C)
+    float* C = nullptr; int ldc = 0; int M = 0, N = 0, K = 0;
+    const float* scale = nullptr; const float* shift = nullptr;
+    float neg_slope = 1.f;   // act(v) = max(v, v * neg_slope), see act_neg_slope
+    int tiles_m = 0, tiles_n = 0;
+    int batch = 1; long long strideC = 0;   // TN: slice z contracts rows [z*K, (z+1)*K) of both operands into C + z*strideC
+    int bM = 0, bN = 0;             // !TN, batch > 1: slice z multiplies rows [z*bM, ..) of A with rows [z*bN, ..) of B into C rows z*bM ..
+    int accumulate = 0;             // !TN: C += result (the epilogue reads C)
     // EPI == 1 (BN == 64): row softmax of the affine result instead of the activation; C (fp32, may be null), a_h (fp16 copy, may
     // be null) and apart[row block of 32][64] = the column sums of every 32-row block (may be null)
-    __half* a_h; float* apart;
+    __half* a_h = nullptr; float* apart = nullptr;
 };
 
 // TN == false:  C[m][n] = sum_k A[m][k] B[n][k]      (both operands K-contiguous: "K-major" UMMA tiles)
@@ -327,30 +326,15 @@ template <int BN, int STAGES, bool TN = false, typename TIN = float, bool OUT_HA
 static int launch(const CUtensorMap& ta, const CUtensorMap& tb, Params p, cudaStream_t st) {
     constexpr size_t smem = (size_t)STAGES * (BM * BK * 4 + BN * BK * 4) + EPI_WARPS * 32 * 32 * 4 + 256 + (EPI == 1 ? 2048 : 0);
     LPD_CUDA_CHECK(allow_smem(gemm_tf32_kernel<BN, STAGES, TN, TIN, OUT_HALF, EPI>, smem));
-    int dev = 0, sms = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    const int rc = sm_count(&sms);
+    if (rc != LPD_OK) return rc;
     p.tiles_m = ceil_div(p.M, BM);
     p.tiles_n = ceil_div(p.N, BN);
     const long long tiles = (long long)p.tiles_m * p.tiles_n * p.batch;
     const int grid = (int)(tiles < sms ? tiles : sms);
     gemm_tf32_kernel<BN, STAGES, TN, TIN, OUT_HALF, EPI><<<grid, THREADS, smem, st>>>(ta, tb, p);
     LPD_LAUNCH_CHECK();
-    return LPD_OK;
-}
-
-// 2-D fp16 tensor [rows][cols] with leading dimension ld (elements), box = [box_rows][64 cols = 128 B], 128B swizzle
-static int make_tmap_h(CUtensorMap* m, const void* base, long long rows, int cols, int ld, int box_rows) {
-    EncodeTiledFn enc = get_encode();
-    if (!enc) { snprintf(g_last_error, sizeof(g_last_error), "cuTensorMapEncodeTiled entry point not found"); return LPD_ECUDA; }
-    cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-    cuuint32_t box[2] = {64u, (cuuint32_t)box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { snprintf(g_last_error, sizeof(g_last_error), "cuTensorMapEncodeTiled (fp16) failed: CUresult %d", (int)r); return LPD_ECUDA; }
     return LPD_OK;
 }
 
@@ -596,9 +580,9 @@ gemm_h2_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
 template <typename TIN, bool OUT32 = false>
 static int launch_h2(const CUtensorMap& ta, const CUtensorMap& tb, Params p, cudaStream_t st) {
     LPD_CUDA_CHECK(allow_smem(gemm_h2_kernel<TIN, OUT32>, H2_SMEM));
-    int dev = 0, sms = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    const int rc = sm_count(&sms);
+    if (rc != LPD_OK) return rc;
     p.tiles_m = ceil_div(p.M, 256);
     p.tiles_n = p.N / 256;
     const long long tiles = (long long)p.tiles_m * p.tiles_n;
@@ -607,6 +591,62 @@ static int launch_h2(const CUtensorMap& ta, const CUtensorMap& tb, Params p, cud
     gemm_h2_kernel<TIN, OUT32><<<grid, THREADS, H2_SMEM, st>>>(ta, tb, p);
     LPD_LAUNCH_CHECK();
     return LPD_OK;
+}
+
+// One validated GEMM of the extern "C" entry points.  !tn: A [batch*M][K], B [batch*N][K]; tn: A [batch*K][M], B [batch*K][N].
+struct GemmCall {
+    const void* A = nullptr; int lda = 0;
+    const void* B = nullptr; int ldb = 0;
+    bool half = false;       // fp16 operands (kind::f16); else fp32 operands read as TF32
+    bool tn = false;
+    bool out_half = false;   // C is fp16
+    bool softmax = false;    // EPI 1: row softmax over N == 64 columns
+    Params p;
+};
+
+// the single-CTA kernel at tile width BN, with as many ring stages as its shared memory holds
+template <typename TIN, bool TN, bool OUT_HALF>
+static int launch_bn(int BN, const CUtensorMap& ta, const CUtensorMap& tb, const Params& p, cudaStream_t st) {
+    if (BN == 64) return launch<64, 8, TN, TIN, OUT_HALF>(ta, tb, p, st);
+    if (BN == 128) return launch<128, 6, TN, TIN, OUT_HALF>(ta, tb, p, st);
+    return launch<256, 4, TN, TIN, OUT_HALF>(ta, tb, p, st);
+}
+
+template <typename TIN>
+static int launch_form(const GemmCall& g, int BN, const CUtensorMap& ta, const CUtensorMap& tb, cudaStream_t st) {
+    if (g.softmax) return launch<64, 8, false, TIN, false, 1>(ta, tb, g.p, st);
+    if (g.tn) return launch_bn<TIN, true, false>(BN, ta, tb, g.p, st);
+    if (g.out_half) return launch_bn<TIN, false, true>(BN, ta, tb, g.p, st);
+    return launch_bn<TIN, false, false>(BN, ta, tb, g.p, st);
+}
+
+static int gemm_run(const GemmCall& g, cudaStream_t st) {
+    int rc = require_sm100();
+    if (rc != LPD_OK) return rc;
+    const Params& p = g.p;
+    // CTA-pair kernel: wide layers whose epilogue scale / shift fit its shared memory, with fp16 output (16-byte row stores) or
+    // as one large fp32 product
+    const bool pair = !g.tn && !g.softmax && (p.N % 256) == 0 && p.N <= H2_MAXN &&
+                      (g.out_half ? (p.ldc % 8) == 0 : !g.half && p.batch == 1 && !p.accumulate && p.M >= 1024);
+    const int BN = p.N <= 64 ? 64 : (p.N <= 128 ? 128 : 256);
+    const CUtensorMapDataType type = g.half ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+    const int row = g.half ? 64 : 32;                       // elements per 128-byte shared-memory row
+    CUtensorMap ta, tb;
+    if (g.tn) {   // boxes {128 bytes along M / N, as many k-rows}; MN-major tf32 needs the 32-byte swizzle atom
+        const long long rows = (long long)p.K * p.batch;
+        const CUtensorMapSwizzle swz = g.half ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B;
+        rc = make_tmap(&ta, type, g.A, rows, p.M, g.lda, row, row, swz);
+        if (rc == LPD_OK) rc = make_tmap(&tb, type, g.B, rows, p.N, g.ldb, row, row, swz);
+    } else {      // a CTA of the pair loads 128 of the 256 rows of B in its tile
+        rc = make_tmap(&ta, type, g.A, (long long)p.batch * p.M, p.K, g.lda, BM, row);
+        if (rc == LPD_OK) rc = make_tmap(&tb, type, g.B, (long long)p.batch * p.N, p.K, g.ldb, pair ? 128 : BN, row);
+    }
+    if (rc != LPD_OK) return rc;
+    if (pair) {
+        if (g.half) return launch_h2<__half>(ta, tb, p, st);
+        return g.out_half ? launch_h2<float>(ta, tb, p, st) : launch_h2<float, true>(ta, tb, p, st);
+    }
+    return g.half ? launch_form<__half>(g, BN, ta, tb, st) : launch_form<float>(g, BN, ta, tb, st);
 }
 
 __global__ void __launch_bounds__(256)
@@ -698,9 +738,6 @@ extern "C" int lpd_f32_to_f16(const float* x, long long ldx, void* y, long long 
     return LPD_OK;
 }
 
-// 1 (default): wide fp16-output layers on the CTA-pair kernel; 0: single-CTA kernel everywhere (LPD_GEMM_2CTA=0)
-static int g_gemm_2cta = [] { const char* e = getenv("LPD_GEMM_2CTA"); return (e && atoi(e) == 0) ? 0 : 1; }();
-
 extern "C" int lpd_gemm_f16(const void* A, int lda, const void* W, int ldw, void* C, int ldc, int out_half,
                             int M, int N, int K, const float* scale, const float* shift, int act, float slope, void* stream) {
     using namespace lpd;
@@ -709,35 +746,12 @@ extern "C" int lpd_gemm_f16(const void* A, int lda, const void* W, int ldw, void
     LPD_REQUIRE((lda % 8) == 0 && (ldw % 8) == 0 && (ldc % 4) == 0);          // 16-byte global strides (TMA), vector stores
     LPD_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)W & 15) == 0 && ((uintptr_t)C & 15) == 0);
     LPD_REQUIRE((N % 4) == 0);
-    LPD_REQUIRE(act == LPD_ACT_NONE || act == LPD_ACT_RELU || (act == LPD_ACT_LEAKY && slope >= 0.f && slope <= 1.f));
-    int dev = 0, major = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
-    if (major != 10) return LPD_EUNSUPPORTED;
-    const int BN = N <= 64 ? 64 : (N <= 128 ? 128 : 256);
-    CUtensorMap ta, tb;
-    int rc = tc::make_tmap_h(&ta, A, M, K, lda, tc::BM);
-    if (rc != LPD_OK) return rc;
-    rc = tc::make_tmap_h(&tb, W, N, K, ldw, BN);
-    if (rc != LPD_OK) return rc;
-    tc::Params p;
-    p.C = reinterpret_cast<float*>(C); p.ldc = ldc; p.M = M; p.N = N; p.K = K; p.scale = scale; p.shift = shift;
-    p.neg_slope = act == LPD_ACT_NONE ? 1.f : (act == LPD_ACT_RELU ? 0.f : slope);
-    p.tiles_m = p.tiles_n = 0; p.batch = 1; p.strideC = 0; p.bM = p.bN = 0; p.accumulate = 0; p.a_h = nullptr; p.apart = nullptr;
-    cudaStream_t st = as_stream(stream);
-    if (out_half && (N % 256) == 0 && N <= tc::H2_MAXN && (ldc % 8) == 0 && g_gemm_2cta) {   // CTA-pair kernel (cta_group::2)
-        rc = tc::make_tmap_h(&tb, W, N, K, ldw, 128);                                  // each CTA loads 128 of the tile's 256 rows of W
-        if (rc != LPD_OK) return rc;
-        return tc::launch_h2<__half>(ta, tb, p, st);
-    }
-    if (out_half) {
-        if (BN == 64) return tc::launch<64, 8, false, __half, true>(ta, tb, p, st);
-        if (BN == 128) return tc::launch<128, 6, false, __half, true>(ta, tb, p, st);
-        return tc::launch<256, 4, false, __half, true>(ta, tb, p, st);
-    }
-    if (BN == 64) return tc::launch<64, 8, false, __half, false>(ta, tb, p, st);
-    if (BN == 128) return tc::launch<128, 6, false, __half, false>(ta, tb, p, st);
-    return tc::launch<256, 4, false, __half, false>(ta, tb, p, st);
+    LPD_REQUIRE(act_is_slope(act, slope));
+    tc::GemmCall g;
+    g.A = A; g.lda = lda; g.B = W; g.ldb = ldw; g.half = true; g.out_half = out_half != 0;
+    g.p.C = reinterpret_cast<float*>(C); g.p.ldc = ldc; g.p.M = M; g.p.N = N; g.p.K = K; g.p.scale = scale; g.p.shift = shift;
+    g.p.neg_slope = act_neg_slope(act, slope);
+    return tc::gemm_run(g, as_stream(stream));
 }
 
 extern "C" int lpd_gemm_f16_tn(const void* A, int lda, const void* B, int ldb, float* C, int ldc, long long strideC,
@@ -749,24 +763,10 @@ extern "C" int lpd_gemm_f16_tn(const void* A, int lda, const void* B, int ldb, f
     LPD_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)B & 15) == 0 && ((uintptr_t)C & 15) == 0);
     LPD_REQUIRE((N % 4) == 0);
     LPD_REQUIRE(batch == 1 || (K % 64) == 0);              // a slice's k-blocks must not run into the next slice
-    int dev = 0, major = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
-    if (major != 10) return LPD_EUNSUPPORTED;
-    const int BN = N <= 64 ? 64 : (N <= 128 ? 128 : 256);
-    const long long rows = (long long)K * batch;
-    CUtensorMap ta, tb;
-    int rc = tc::make_tmap_h(&ta, A, rows, M, lda, 64);     // boxes {64 halves along M, 64 k-rows}
-    if (rc != LPD_OK) return rc;
-    rc = tc::make_tmap_h(&tb, B, rows, N, ldb, 64);
-    if (rc != LPD_OK) return rc;
-    tc::Params p;
-    p.C = C; p.ldc = ldc; p.M = M; p.N = N; p.K = K; p.scale = nullptr; p.shift = nullptr; p.neg_slope = 1.f;
-    p.tiles_m = p.tiles_n = 0; p.batch = batch; p.strideC = strideC; p.bM = p.bN = 0; p.accumulate = 0; p.a_h = nullptr; p.apart = nullptr;
-    cudaStream_t st = as_stream(stream);
-    if (BN == 64) return tc::launch<64, 8, true, __half>(ta, tb, p, st);
-    if (BN == 128) return tc::launch<128, 6, true, __half>(ta, tb, p, st);
-    return tc::launch<256, 4, true, __half>(ta, tb, p, st);
+    tc::GemmCall g;
+    g.A = A; g.lda = lda; g.B = B; g.ldb = ldb; g.half = true; g.tn = true;
+    g.p.C = C; g.p.ldc = ldc; g.p.M = M; g.p.N = N; g.p.K = K; g.p.batch = batch; g.p.strideC = strideC;
+    return tc::gemm_run(g, as_stream(stream));
 }
 
 extern "C" int lpd_gemm_tf32_ex(const float* A, int lda, const float* B, int ldb, float* C, int ldc,
@@ -778,32 +778,14 @@ extern "C" int lpd_gemm_tf32_ex(const float* A, int lda, const float* B, int ldb
     LPD_REQUIRE((lda % 4) == 0 && (ldb % 4) == 0 && (ldc % 4) == 0);          // 16-byte global strides (TMA) / float4 stores
     LPD_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)B & 15) == 0 && ((uintptr_t)C & 15) == 0);
     LPD_REQUIRE((N % 4) == 0);
-    LPD_REQUIRE(act == LPD_ACT_NONE || act == LPD_ACT_RELU || (act == LPD_ACT_LEAKY && slope >= 0.f && slope <= 1.f));
+    LPD_REQUIRE(act_is_slope(act, slope));
     LPD_REQUIRE((long long)batch * M < (1ll << 31) && (long long)batch * N < (1ll << 31));
-    int dev = 0, major = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
-    if (major != 10) return LPD_EUNSUPPORTED;
-    const int BN = N <= 64 ? 64 : (N <= 128 ? 128 : 256);
-    CUtensorMap ta, tb;
-    int rc = tc::make_tmap(&ta, A, (long long)batch * M, K, lda, tc::BM);
-    if (rc != LPD_OK) return rc;
-    rc = tc::make_tmap(&tb, B, (long long)batch * N, K, ldb, BN);
-    if (rc != LPD_OK) return rc;
-    tc::Params p;
-    p.C = C; p.ldc = ldc; p.M = M; p.N = N; p.K = K; p.scale = scale; p.shift = shift;
-    p.neg_slope = act == LPD_ACT_NONE ? 1.f : (act == LPD_ACT_RELU ? 0.f : slope);
-    p.tiles_m = p.tiles_n = 0; p.batch = batch; p.strideC = 0;
-    p.bM = batch > 1 ? M : 0; p.bN = batch > 1 ? N : 0; p.accumulate = accumulate ? 1 : 0; p.a_h = nullptr; p.apart = nullptr;
-    cudaStream_t st = as_stream(stream);
-    if (batch == 1 && !accumulate && (N % 256) == 0 && N <= tc::H2_MAXN && M >= 1024 && g_gemm_2cta) {   // CTA-pair kernel, fp32 output
-        rc = tc::make_tmap(&tb, B, N, K, ldb, 128);
-        if (rc != LPD_OK) return rc;
-        return tc::launch_h2<float, true>(ta, tb, p, st);
-    }
-    if (BN == 64) return tc::launch<64, 8>(ta, tb, p, st);
-    if (BN == 128) return tc::launch<128, 6>(ta, tb, p, st);
-    return tc::launch<256, 4>(ta, tb, p, st);
+    tc::GemmCall g;
+    g.A = A; g.lda = lda; g.B = B; g.ldb = ldb;
+    g.p.C = C; g.p.ldc = ldc; g.p.M = M; g.p.N = N; g.p.K = K; g.p.scale = scale; g.p.shift = shift;
+    g.p.neg_slope = act_neg_slope(act, slope);
+    g.p.batch = batch; g.p.bM = batch > 1 ? M : 0; g.p.bN = batch > 1 ? N : 0; g.p.accumulate = accumulate ? 1 : 0;
+    return tc::gemm_run(g, as_stream(stream));
 }
 
 extern "C" int lpd_gemm_tf32_out16(const float* A, int lda, const float* B, int ldb, void* C, int ldc, int M, int N, int K,
@@ -813,30 +795,12 @@ extern "C" int lpd_gemm_tf32_out16(const float* A, int lda, const float* B, int 
     LPD_REQUIRE(lda >= K && ldb >= K && ldc >= N);
     LPD_REQUIRE((lda % 4) == 0 && (ldb % 4) == 0 && (ldc % 4) == 0 && (N % 4) == 0);
     LPD_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)B & 15) == 0 && ((uintptr_t)C & 7) == 0);
-    LPD_REQUIRE(act == LPD_ACT_NONE || act == LPD_ACT_RELU || (act == LPD_ACT_LEAKY && slope >= 0.f && slope <= 1.f));
-    int dev = 0, major = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
-    if (major != 10) return LPD_EUNSUPPORTED;
-    const int BN = N <= 64 ? 64 : (N <= 128 ? 128 : 256);
-    CUtensorMap ta, tb;
-    int rc = tc::make_tmap(&ta, A, M, K, lda, tc::BM);
-    if (rc != LPD_OK) return rc;
-    rc = tc::make_tmap(&tb, B, N, K, ldb, BN);
-    if (rc != LPD_OK) return rc;
-    tc::Params p;
-    p.C = reinterpret_cast<float*>(C); p.ldc = ldc; p.M = M; p.N = N; p.K = K; p.scale = scale; p.shift = shift;
-    p.neg_slope = act == LPD_ACT_NONE ? 1.f : (act == LPD_ACT_RELU ? 0.f : slope);
-    p.tiles_m = p.tiles_n = 0; p.batch = 1; p.strideC = 0; p.bM = p.bN = 0; p.accumulate = 0; p.a_h = nullptr; p.apart = nullptr;
-    cudaStream_t st = as_stream(stream);
-    if ((N % 256) == 0 && N <= tc::H2_MAXN && (ldc % 8) == 0 && g_gemm_2cta) {         // CTA-pair kernel (cta_group::2)
-        rc = tc::make_tmap(&tb, B, N, K, ldb, 128);
-        if (rc != LPD_OK) return rc;
-        return tc::launch_h2<float>(ta, tb, p, st);
-    }
-    if (BN == 64) return tc::launch<64, 8, false, float, true>(ta, tb, p, st);
-    if (BN == 128) return tc::launch<128, 6, false, float, true>(ta, tb, p, st);
-    return tc::launch<256, 4, false, float, true>(ta, tb, p, st);
+    LPD_REQUIRE(act_is_slope(act, slope));
+    tc::GemmCall g;
+    g.A = A; g.lda = lda; g.B = B; g.ldb = ldb; g.out_half = true;
+    g.p.C = reinterpret_cast<float*>(C); g.p.ldc = ldc; g.p.M = M; g.p.N = N; g.p.K = K; g.p.scale = scale; g.p.shift = shift;
+    g.p.neg_slope = act_neg_slope(act, slope);
+    return tc::gemm_run(g, as_stream(stream));
 }
 
 extern "C" int lpd_gemm_tf32(const float* A, int lda, const float* B, int ldb, float* C, int ldc,
@@ -854,24 +818,10 @@ extern "C" int lpd_gemm_tf32_tn(const float* A, int lda, const float* B, int ldb
     LPD_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)B & 15) == 0 && ((uintptr_t)C & 15) == 0);
     LPD_REQUIRE((N % 4) == 0);
     LPD_REQUIRE(batch == 1 || (K % tc::BK) == 0);          // a slice's k-blocks must not run into the next slice
-    int dev = 0, major = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
-    if (major != 10) return LPD_EUNSUPPORTED;
-    const int BN = N <= 64 ? 64 : (N <= 128 ? 128 : 256);
-    const long long rows = (long long)K * batch;
-    CUtensorMap ta, tb;
-    int rc = tc::make_tmap(&ta, A, rows, M, lda, 32, true); // boxes {32 floats along M, 32 k-rows}, 32-byte swizzle atom
-    if (rc != LPD_OK) return rc;
-    rc = tc::make_tmap(&tb, B, rows, N, ldb, 32, true);
-    if (rc != LPD_OK) return rc;
-    tc::Params p;
-    p.C = C; p.ldc = ldc; p.M = M; p.N = N; p.K = K; p.scale = nullptr; p.shift = nullptr; p.neg_slope = 1.f;
-    p.tiles_m = p.tiles_n = 0; p.batch = batch; p.strideC = strideC; p.bM = p.bN = 0; p.accumulate = 0; p.a_h = nullptr; p.apart = nullptr;
-    cudaStream_t st = as_stream(stream);
-    if (BN == 64) return tc::launch<64, 8, true>(ta, tb, p, st);
-    if (BN == 128) return tc::launch<128, 6, true>(ta, tb, p, st);
-    return tc::launch<256, 4, true>(ta, tb, p, st);
+    tc::GemmCall g;
+    g.A = A; g.lda = lda; g.B = B; g.ldb = ldb; g.tn = true;
+    g.p.C = C; g.p.ldc = ldc; g.p.M = M; g.p.N = N; g.p.K = K; g.p.batch = batch; g.p.strideC = strideC;
+    return tc::gemm_run(g, as_stream(stream));
 }
 
 extern "C" int lpd_gemm_softmax64(const void* A, int a_f16, int lda, const void* W, int ldw, int M, int K, const float* scale,
@@ -883,20 +833,9 @@ extern "C" int lpd_gemm_softmax64(const void* A, int a_f16, int lda, const void*
     LPD_REQUIRE((lda % al) == 0 && (ldw % al) == 0);
     LPD_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)W & 15) == 0 && ((uintptr_t)a32 & 15) == 0 && ((uintptr_t)a16 & 7) == 0 &&
                 ((uintptr_t)apart & 15) == 0);
-    int dev = 0, major = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
-    if (major != 10) return LPD_EUNSUPPORTED;
-    CUtensorMap ta, tb;
-    int rc = a_f16 ? tc::make_tmap_h(&ta, A, M, K, lda, tc::BM) : tc::make_tmap(&ta, reinterpret_cast<const float*>(A), M, K, lda, tc::BM);
-    if (rc != LPD_OK) return rc;
-    rc = a_f16 ? tc::make_tmap_h(&tb, W, 64, K, ldw, 64) : tc::make_tmap(&tb, reinterpret_cast<const float*>(W), 64, K, ldw, 64);
-    if (rc != LPD_OK) return rc;
-    tc::Params p;
-    p.C = a32; p.ldc = 64; p.M = M; p.N = 64; p.K = K; p.scale = scale; p.shift = shift; p.neg_slope = 1.f;
-    p.tiles_m = p.tiles_n = 0; p.batch = 1; p.strideC = 0; p.bM = p.bN = 0; p.accumulate = 0;
-    p.a_h = reinterpret_cast<__half*>(a16); p.apart = apart;
-    cudaStream_t st = as_stream(stream);
-    if (a_f16) return tc::launch<64, 8, false, __half, false, 1>(ta, tb, p, st);
-    return tc::launch<64, 8, false, float, false, 1>(ta, tb, p, st);
+    tc::GemmCall g;
+    g.A = A; g.lda = lda; g.B = W; g.ldb = ldw; g.half = a_f16 != 0; g.softmax = true;
+    g.p.C = a32; g.p.ldc = 64; g.p.M = M; g.p.N = 64; g.p.K = K; g.p.scale = scale; g.p.shift = shift;
+    g.p.a_h = reinterpret_cast<__half*>(a16); g.p.apart = apart;
+    return tc::gemm_run(g, as_stream(stream));
 }

@@ -388,9 +388,9 @@ template <int GS, int QD>
 static int knn_tc_launch(const CUtensorMap& ta, const CUtensorMap& tb, const KnnTcParams& P, cudaStream_t st) {
     const size_t smem = KtSmem<GS, QD>::total;
     LPD_CUDA_CHECK(allow_smem(knn_tc_kernel<GS, QD>, smem));
-    int dev = 0, sms = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    const int rc = sm_count(&sms);
+    if (rc != LPD_OK) return rc;
     const int items = P.B * P.qtiles;
     knn_tc_kernel<GS, QD><<<items < sms ? items : sms, KT_THREADS, smem, st>>>(ta, tb, P);
     LPD_LAUNCH_CHECK();
@@ -455,10 +455,8 @@ extern "C" int lpd_knn_tc(const float* x, int B, int N, int C, int k, void* idx,
     LPD_REQUIRE(((uintptr_t)x & 15) == 0 && ((uintptr_t)workspace & 255) == 0);
     const tc::KnnWs W(B, N, k);
     if (workspace_bytes < lpd_knn_workspace_bytes(B, N, C, k)) return LPD_EWORKSPACE;
-    int dev = 0, major = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&major, cudaDevAttrComputeCapabilityMajor, dev));
-    if (major != 10) return LPD_EUNSUPPORTED;
+    int rc = require_sm100();
+    if (rc != LPD_OK) return rc;
     cudaStream_t st = as_stream(stream);
     if (tc::g_knn_variant != 0) return tc::knn2_run(x, B, N, k, idx, idx_i64, workspace, workspace_bytes, tc::g_knn_variant, st);
     uint8_t* ws = reinterpret_cast<uint8_t*>(workspace);
@@ -472,9 +470,9 @@ extern "C" int lpd_knn_tc(const float* x, int B, int N, int C, int k, void* idx,
     tc::knn_split_kernel<<<dim3(ceil_div(W.npad, 256), B), 256, 0, st>>>(x, N, W.npad, x2, xxpad, r2);
     LPD_LAUNCH_CHECK();
     CUtensorMap ta, tb;
-    int rc = tc::make_tmap(&ta, x2, (long long)B * N, 128, 128, tc::KT_Q);
+    rc = tc::make_tmap(&ta, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, x2, (long long)B * N, 128, 128, tc::KT_Q, 32);
     if (rc != LPD_OK) return rc;
-    rc = tc::make_tmap(&tb, x2, (long long)B * N, 128, 128, tc::KT_C);
+    rc = tc::make_tmap(&tb, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, x2, (long long)B * N, 128, 128, tc::KT_C, 32);
     if (rc != LPD_OK) return rc;
     tc::KnnTcParams P;
     P.xxpad = xxpad;

@@ -1048,15 +1048,15 @@ template <int CAP, int WARPS>
 static int knn2_refine_tma_launch(const float* x, const float* xxpad, const int* cnt, const int* cand, int B, int N, int Npad, int k,
                                   void* idx, int idx_i64, int* flags, int* list, cudaStream_t st) {
     CUtensorMap tx;
-    int rc = make_tmap(&tx, x, (long long)B * N, 64, 64, 1);          // box = one half row (32 floats = 128 B), 128B swizzle
+    // box = one half row (32 floats = 128 B), 128B swizzle
+    int rc = make_tmap(&tx, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, x, (long long)B * N, 64, 64, 1, 32);
     if (rc != LPD_OK) return rc;
     const size_t smem = RefineTmaSmem<CAP, WARPS>::total;
     static int sms = 0, per_sm = 0;                                   // per instantiation; one device model per process
     if (per_sm == 0) {
-        int dev = 0;
         LPD_CUDA_CHECK(allow_smem(knn2_refine_tma_kernel<CAP, WARPS>, smem));
-        LPD_CUDA_CHECK(cudaGetDevice(&dev));
-        LPD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+        rc = sm_count(&sms);
+        if (rc != LPD_OK) return rc;
         LPD_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, knn2_refine_tma_kernel<CAP, WARPS>, WARPS * 32, smem));
         if (per_sm < 1) per_sm = 1;
     }
@@ -1084,21 +1084,6 @@ static int knn2_refine_launch(const float* x, const float* xxpad, const int* cnt
     const unsigned rblocks = (unsigned)(((long long)B * N + RF_WARPS - 1) / RF_WARPS);
     knn2_refine_kernel<CAP><<<rblocks, RF_WARPS * 32, smem, st>>>(x, xxpad, cnt, cand, B, N, Npad, k, idx, idx_i64, flags, list);
     LPD_LAUNCH_CHECK();
-    return LPD_OK;
-}
-
-// 2-D fp16 tensor [rows][64], box = [box_rows][64 cols = 128 B], 128B swizzle
-static int make_tmap_f16(CUtensorMap* m, const __half* base, long long rows, int box_rows) {
-    EncodeTiledFn enc = get_encode();
-    if (!enc) { snprintf(g_last_error, sizeof(g_last_error), "cuTensorMapEncodeTiled entry point not found"); return LPD_ECUDA; }
-    cuuint64_t dims[2] = {64u, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {128u};
-    cuuint32_t box[2] = {64u, (cuuint32_t)box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 2, const_cast<__half*>(base), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) { snprintf(g_last_error, sizeof(g_last_error), "cuTensorMapEncodeTiled (fp16) failed: CUresult %d", (int)r); return LPD_ECUDA; }
     return LPD_OK;
 }
 
@@ -1140,9 +1125,9 @@ template <int MT, int CAP, bool TIGHT, bool TS = false>
 static int knn2_launch(const CUtensorMap& ta, const CUtensorMap& tb, const Knn2Params& P, cudaStream_t st) {
     const size_t smem = K2Smem<MT, TS>::total;
     LPD_CUDA_CHECK(allow_smem(knn2_tc_kernel<MT, CAP, TIGHT, TS>, smem));
-    int dev = 0, sms = 0;
-    LPD_CUDA_CHECK(cudaGetDevice(&dev));
-    LPD_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 0;
+    const int rc = sm_count(&sms);
+    if (rc != LPD_OK) return rc;
     const int items = P.B * P.qtiles;
     knn2_tc_kernel<MT, CAP, TIGHT, TS><<<items < sms ? items : sms, 256 * MT + 64, smem, st>>>(ta, tb, P);
     LPD_LAUNCH_CHECK();
@@ -1173,10 +1158,10 @@ int knn2_run(const float* x, int B, int N, int k, void* idx, int idx_i64, void* 
     if (!prep_smem_ok) { LPD_CUDA_CHECK(allow_smem(knn2_prep_kernel, K2_PREP_SMEM)); prep_smem_ok = true; }
     knn2_prep_kernel<<<dim3(ceil_div(W.npad, 256), B), 256, K2_PREP_SMEM, st>>>(x, mu, sc, N, W.npad, xh, reinterpret_cast<uint4*>(ws + W.off_ext), xxpad, nrmpad, snpad, r2, r2c);
     LPD_LAUNCH_CHECK();
-    CUtensorMap ta, tb;
-    int rc = make_tmap_f16(&ta, xh, (long long)B * N, 128);
+    CUtensorMap ta, tb;   // xh fp16 [B*N][64]: boxes of 128 query rows / K2_C = 128 candidates per stage, 64 halves each
+    int rc = make_tmap(&ta, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, xh, (long long)B * N, 64, 64, 128, 64);
     if (rc != LPD_OK) return rc;
-    rc = make_tmap_f16(&tb, xh, (long long)B * N, K2_C);      // 128 candidates per stage
+    rc = make_tmap(&tb, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, xh, (long long)B * N, 64, 64, K2_C, 64);
     if (rc != LPD_OK) return rc;
     Knn2Params P;
     P.nrmpad = nrmpad; P.snpad = snpad; P.ext = reinterpret_cast<const uint4*>(ws + W.off_ext); P.xh = reinterpret_cast<const uint4*>(xh); P.xxpad = xxpad; P.r2 = r2; P.r2c = r2c; P.sc = sc;

@@ -116,8 +116,8 @@ extern "C" int lpd_pointwise_mlp2(const float* x, int ldx, int D, long long M, c
     using namespace lpd;
     LPD_REQUIRE(x && w1 && s1 && t1 && w2 && s2 && t2 && out && M >= 1);
     LPD_REQUIRE(D >= 1 && D <= PW_MAXD && ldx >= D && ldo >= 64);
-    LPD_REQUIRE(act == LPD_ACT_NONE || act == LPD_ACT_RELU || (act == LPD_ACT_LEAKY && slope >= 0.f && slope <= 1.f));
-    const float neg_slope = act == LPD_ACT_NONE ? 1.f : (act == LPD_ACT_RELU ? 0.f : slope);
+    LPD_REQUIRE(act_is_slope(act, slope));
+    const float neg_slope = act_neg_slope(act, slope);
     long long blocks = (M + PW_THREADS - 1) / PW_THREADS;
     if (blocks > 148 * 3) blocks = 148 * 3;                   // persistent: three resident blocks per SM (register-bound), W2 loaded once per thread
     pointwise_mlp2_kernel<<<(int)blocks, PW_THREADS, 0, as_stream(stream)>>>(x, ldx, D, M, w1, s1, t1, w2, s2, t2, neg_slope, out, ldo);

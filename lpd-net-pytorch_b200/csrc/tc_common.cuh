@@ -165,18 +165,19 @@ inline EncodeTiledFn get_encode() {
     return fn;
 }
 
-// 2-D fp32 tensor [rows][cols] with leading dimension ld (elements), box = [box_rows][32 cols], 128B swizzle
-inline int make_tmap(CUtensorMap* m, const float* base, long long rows, int cols, int ld, int box_rows, bool atom32 = false) {
+// 2-D tensor [rows][cols] of fp32 or fp16 (type) with row pitch ld (elements), loaded in boxes of box_rows x box_cols;
+// out-of-range box elements read as zero
+inline int make_tmap(CUtensorMap* m, CUtensorMapDataType type, const void* base, long long rows, long long cols, long long ld,
+                     int box_rows, int box_cols, CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
     EncodeTiledFn enc = get_encode();
     if (!enc) { snprintf(g_last_error, sizeof(g_last_error), "cuTensorMapEncodeTiled entry point not found"); return LPD_ECUDA; }
+    const size_t esize = type == CU_TENSOR_MAP_DATA_TYPE_FLOAT16 ? 2 : 4;
     cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)ld * sizeof(float)};
-    cuuint32_t box[2] = {32u, (cuuint32_t)box_rows};
+    cuuint64_t strides[1] = {(cuuint64_t)ld * esize};
+    cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
     cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(base), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, atom32 ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B,
-                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    CUresult r = enc(m, type, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle,
+                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { snprintf(g_last_error, sizeof(g_last_error), "cuTensorMapEncodeTiled failed: CUresult %d", (int)r); return LPD_ECUDA; }
     return LPD_OK;
 }
