@@ -203,7 +203,9 @@ int lpd_gemm_tf32_out16(const float* A, int lda, const float* B, int ldb, void* 
 /* lpd_softmax64 that also writes the probabilities as fp16 (a_h [M][64]): the B operand of the f16-mode NetVLAD aggregate. */
 int lpd_softmax64_f16(float* a, long long M, void* a_h, void* stream);
 /* f16-mode forms of the pre-scaled edge kernels (fp16 rows in and out, see lpd_edge_gather_ext / lpd_edgeconv_dg_tf32):
- *   lpd_edge_gather_max_f16:  out[i][:] = act(q[i][:] + max_m p[j(i,m)][:]),  C == 256            (csrc/edge.cu)
+ *   lpd_edge_gather_max_f16:  out[i][:] = act(q[i][:] + max_m p[j(i,m)][:]),  C == 256 or 64     (csrc/edge.cu)
+ *                             (C == 64 with q == NULL, ACT_NONE: LPDNetOrign's gather-only SN stage, reference
+ *                             lpdnet_model.py:104, :144)
  *   lpd_edgeconv_dg20_f16:    k == 20, 128 channels; y1 = act(p_j + q_i) and W2 in fp16, second layer on tcgen05 kind::f16,
  *                             x1 / x2 written as fp16                                             (csrc/edge_tc20.cu) */
 int lpd_edge_gather_max_f16(const void* p, int ldp, const void* q, int ldq, const int32_t* idx, int B, int N, int k, int C,
@@ -215,6 +217,17 @@ int lpd_edgeconv_dg20_f16(const void* p, int ldp, const void* q, int ldq, const 
 int lpd_edgeconv_dg32_f16(const void* p, int ldp, const void* q, int ldq, const int32_t* idx, int B, int N,
                           const void* w2, const float* s2, const float* t2, int act, float slope,
                           void* x1, int ld1, void* x2, int ld2, void* stream);
+/* LPDNetOrign's convDG1 + convDG2 + max (reference lpdnet_model.py:98-107), f16 mode, 64 channels, k == 20 or 32 (any other k:
+ * LPD_EINVAL, no launch).  The edge [f_i ; f_j - f_i] is decomposed as P = Wb f_j, Q = (Wa - Wb) f_i, and DG1's folded BatchNorm is
+ * carried by p' = s1 P and q' = s1 Q + t1 (fp16 [B*N][ldp] / [B*N][ldq], ldp, ldq % 8 == 0, 16-byte aligned: lpd_gemm_tf32_out16
+ * with epilogue vectors [s1 | s1], [0 | t1]).  Per edge y1 = act(p'_j + q'_i) in fp16, z = W2 y1 on tcgen05 kind::f16 with fp32
+ * accumulation (W2 fp16 [64][64] row-major, 16-byte aligned), then
+ *     x2[i][c] = max_m act(s2[c] z_m[c] + t2[c])            (the min over m is taken where s2[c] < 0)
+ * written as fp16 to x2 [B*N][ld2] (ld2 >= 64 and even).  act in {NONE, RELU, LEAKY with 0 <= slope <= 1}.  No allocation, no host
+ * synchronisation: capturable into a CUDA graph. */
+int lpd_edgeconv_dg64_f16(const void* p, int ldp, const void* q, int ldq, const int32_t* idx, int B, int N, int k,
+                          const void* w2, const float* s2, const float* t2, int act, float slope,
+                          void* x2, int ld2, void* stream);
 
 /* Fused input layers of the LPD-Net feature nets (lpdnet_model.py:231-232, :86-87), strict fp32, one pass:
  *     out[m][:] = act(s2 * (W2 . act(s1 * (W1 . x[m][0..D)) + t1)) + t2),   W1 [64][D], W2 [64][64], D <= 8

@@ -54,6 +54,7 @@ SIGNATURES = {
     "lpd_edge_gather_max_f16": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _f, _vp, _i, _vp]),
     "lpd_edgeconv_dg20_f16": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _vp, _vp, _vp, _i, _f, _vp, _i, _vp, _i, _vp]),
     "lpd_edgeconv_dg32_f16": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _vp, _vp, _vp, _i, _f, _vp, _i, _vp, _i, _vp]),
+    "lpd_edgeconv_dg64_f16": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _vp, _vp, _vp, _i, _f, _vp, _i, _vp]),
     "lpd_pointwise_mlp2": (_i, [_vp, _i, _i, _ll, _vp, _vp, _vp, _vp, _vp, _vp, _i, _f, _vp, _i, _vp]),
     "lpd_colmax": (_i, [_vp, _i, _i, _i, _i, _vp, _vp]),
     "lpd_edge_gather_ext": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _i, _f, _vp, _i, _vp]),

@@ -201,25 +201,29 @@ edge_gather_max_kernel(const float* __restrict__ p, int ldp, const float* __rest
 // per lane and row — half the bytes of the fp32 form through the L1 / L2 data path, which is what bounds this kernel).  The max
 // over the neighbours is taken on the fp16 values directly (exact), the centre term and the activation in fp32, one rounding
 // to nearest on the way out.
+// C = 64 (128-byte rows, LPDNetOrign's gather-only SN stage): 8 lanes cover a row, so the warp's four lane groups load four
+// neighbour rows side by side (group g takes neighbours g, g + 4, ...) and combine their maxima with two shuffles.
 // ------------------------------------------------------------------------------------------------
+template <int C>
 __global__ void __launch_bounds__(256)
 edge_gather_max_h_kernel(const __half* __restrict__ p, int ldp, const __half* __restrict__ q, int ldq,
                          const int* __restrict__ idx, long long total_pts, int N, int k, int act, float slope,
                          __half* __restrict__ out, int ldo) {
-    const int lane = threadIdx.x & 31;
+    constexpr int LPR = C / 8, G = 32 / LPR;         // lanes per row, rows per warp-wide load
+    const int lane = threadIdx.x & 31, g = lane / LPR, col = (lane % LPR) * 8;
     const long long pt = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
     if (pt >= total_pts) return;
     const int myj = lane < k ? __ldg(idx + pt * k + lane) : 0;
-    const __half* base = p + (pt / N) * N * ldp + lane * 8;
-    const uint4 qraw = q ? __ldg(reinterpret_cast<const uint4*>(q + pt * ldq + lane * 8)) : make_uint4(0u, 0u, 0u, 0u);
+    const __half* base = p + (pt / N) * N * ldp + col;
+    const uint4 qraw = q ? __ldg(reinterpret_cast<const uint4*>(q + pt * ldq + col)) : make_uint4(0u, 0u, 0u, 0u);
     const __half2 ninf = __float2half2_rn(-INFINITY);
     __half2 mx[4] = {ninf, ninf, ninf, ninf};
     int m = 0;
-    for (; m + 5 <= k; m += 5) {                     // 5 rows in flight per lane
+    for (; m + 5 * G <= k; m += 5 * G) {             // 5 rows in flight per lane
         uint4 r[5];
 #pragma unroll
         for (int u = 0; u < 5; ++u) {
-            const int j = __shfl_sync(0xffffffffu, myj, m + u);
+            const int j = __shfl_sync(0xffffffffu, myj, m + u * G + g);
             r[u] = __ldg(reinterpret_cast<const uint4*>(base + (unsigned)(j * ldp)));
         }
 #pragma unroll
@@ -229,13 +233,23 @@ edge_gather_max_h_kernel(const __half* __restrict__ p, int ldp, const __half* __
             for (int v = 0; v < 4; ++v) mx[v] = __hmax2(mx[v], h[v]);
         }
     }
-    for (; m < k; ++m) {
-        const int j = __shfl_sync(0xffffffffu, myj, m);
-        const uint4 r = __ldg(reinterpret_cast<const uint4*>(base + (unsigned)(j * ldp)));
-        const __half2* h = reinterpret_cast<const __half2*>(&r);
+    for (; m < k; m += G) {
+        const int mm = m + g;
+        const int j = __shfl_sync(0xffffffffu, myj, mm < k ? mm : m);
+        if (mm < k) {
+            const uint4 r = __ldg(reinterpret_cast<const uint4*>(base + (unsigned)(j * ldp)));
+            const __half2* h = reinterpret_cast<const __half2*>(&r);
 #pragma unroll
-        for (int v = 0; v < 4; ++v) mx[v] = __hmax2(mx[v], h[v]);
+            for (int v = 0; v < 4; ++v) mx[v] = __hmax2(mx[v], h[v]);
+        }
     }
+#pragma unroll
+    for (int off = LPR; off < 32; off <<= 1)
+#pragma unroll
+        for (int v = 0; v < 4; ++v) {
+            const uint32_t o = __shfl_xor_sync(0xffffffffu, *reinterpret_cast<const uint32_t*>(&mx[v]), off);
+            mx[v] = __hmax2(mx[v], *reinterpret_cast<const __half2*>(&o));
+        }
     const __half2* qh = reinterpret_cast<const __half2*>(&qraw);
     uint4 o;
     __half2* oh = reinterpret_cast<__half2*>(&o);
@@ -244,7 +258,7 @@ edge_gather_max_h_kernel(const __half* __restrict__ p, int ldp, const __half* __
         const float2 a = __half22float2(mx[v]), b = __half22float2(qh[v]);
         oh[v] = __floats2half2_rn(act2(a.x + b.x, act, slope), act2(a.y + b.y, act, slope));
     }
-    *reinterpret_cast<uint4*>(out + pt * ldo + lane * 8) = o;
+    if (g == 0) *reinterpret_cast<uint4*>(out + pt * ldo + col) = o;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -415,7 +429,7 @@ extern "C" int lpd_edge_gather_max_f16(const void* p, int ldp, const void* q, in
                                        int act, float slope, void* out, int ldo, void* stream) {
     using namespace lpd;
     LPD_REQUIRE(p && idx && out && B >= 1 && N >= 1 && k >= 1 && k <= 32 && k <= N);
-    LPD_REQUIRE(C == 256);
+    LPD_REQUIRE(C == 256 || C == 64);
     LPD_REQUIRE(ldp % 8 == 0 && ldo % 8 == 0 && ldp >= C && ldo >= C && (!q || (ldq % 8 == 0 && ldq >= C)));
     LPD_REQUIRE(act == LPD_ACT_NONE || act == LPD_ACT_RELU || act == LPD_ACT_LEAKY);
     LPD_REQUIRE(((uintptr_t)p & 15) == 0 && ((uintptr_t)out & 15) == 0 && ((uintptr_t)q & 15) == 0);
@@ -423,7 +437,8 @@ extern "C" int lpd_edge_gather_max_f16(const void* p, int ldp, const void* q, in
     const long long total = (long long)B * N;
     const long long blocks = (total + 7) / 8;
     LPD_REQUIRE(blocks <= 0x7fffffffLL);
-    edge_gather_max_h_kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(
+    auto kernel = C == 256 ? edge_gather_max_h_kernel<256> : edge_gather_max_h_kernel<64>;
+    kernel<<<(unsigned)blocks, 256, 0, as_stream(stream)>>>(
         reinterpret_cast<const __half*>(p), ldp, reinterpret_cast<const __half*>(q), ldq, idx, total, N, k, act, slope,
         reinterpret_cast<__half*>(out), ldo);
     LPD_LAUNCH_CHECK();

@@ -235,9 +235,11 @@ edgeconv_dg20_tc_kernel(const __grid_constant__ CUtensorMap tmap_w2, Dg20Params 
 // runs on tcgen05 kind::f16 (fp32 accumulation).  A gathered row is 256 bytes instead of 512, an operand tile 32 KB instead of
 // 64, and the first layer is three half2 instructions per two values (add, multiply by the slope, max).  Same roles: 4 epilogue
 // warps + 2 groups of 10 producer warps (two per point, one 64-channel k-block each, FOUR rows per warp iteration).
+// C = 64 (LPDNetOrign convDG2, reference util/lpdnet_model.py:98-107): one k-block, so ONE producer warp per point, and W2 is
+// padded with zero rows to the M = 128 accumulator layout of the 128-channel form (TMEM lane = output channel): only epilogue
+// warps 0 and 1 own output channels.  The padded half of each MMA is wasted, but the tensor pipe is not what bounds the kernel.
 // ---------------------------------------------------------------------------------------------------------------------
 constexpr uint32_t D20H_KB_BYTES = 128 * 128;          // one 64-channel k-block of a 128-row fp16 operand tile
-constexpr uint32_t D20H_OP_BYTES = 2 * D20H_KB_BYTES;  // 32 KB
 
 struct Dg20hParams {
     const __half* p; const __half* q; const int* idx;
@@ -249,19 +251,26 @@ struct Dg20hParams {
     long long num_tiles;
 };
 
-// KK = 20: 5 points x 24-row slots per 128-edge tile (the reference's k); KK = 32: 4 points x 32-row slots (the C5 stress shape)
-template <int KK>
+// KK = 20: 5 points x 24-row slots per 128-edge tile (the reference's k); KK = 32: 4 points x 32-row slots (the C5 stress shape).
+// C = 128 or 64 channels in and out.
+template <int KK, int C>
 struct DgH {
-    static constexpr int SLOT = (KK + 7) / 8 * 8, PTS = 128 / SLOT, GROUP_WARPS = 2 * PTS, PROD_WARPS = 2 * GROUP_WARPS;
+    static constexpr int KBS = C / 64;                 // 64-channel k-blocks = producer warps per point
+    static constexpr int SLOT = (KK + 7) / 8 * 8, PTS = 128 / SLOT, GROUP_WARPS = KBS * PTS, PROD_WARPS = 2 * GROUP_WARPS;
     static constexpr int THREADS = 32 * (D20_EPI_WARPS + PROD_WARPS), ROWQ = KK / 4;
+    static constexpr int EPI_LIVE = C / 32;            // epilogue warps that own output channels
+    static constexpr uint32_t OP_BYTES = KBS * D20H_KB_BYTES;
     static_assert(KK % 4 == 0 && KK <= 32 && PTS * SLOT <= 128, "edge tile geometry");
+    static_assert(C == 64 || C == 128, "channel count");
 };
 
-template <int KK>
-__global__ void __launch_bounds__(DgH<KK>::THREADS, 1)
+template <int KK, int C>
+__global__ void __launch_bounds__(DgH<KK, C>::THREADS, 1)
 edgeconv_dg20_h_kernel(const __grid_constant__ CUtensorMap tmap_w2, Dg20hParams P) {
     extern __shared__ __align__(1024) uint8_t smem[];
     if ((smem_u32(smem) & 1023u) != 0) __trap();
+    constexpr uint32_t D20H_OP_BYTES = DgH<KK, C>::OP_BYTES;
+    constexpr int KBS = DgH<KK, C>::KBS, EPI_LIVE = DgH<KK, C>::EPI_LIVE;
     uint8_t* w_s = smem;
     uint8_t* y_s = smem + D20H_OP_BYTES;              // [2][OP_BYTES]
     uint64_t* wfull = reinterpret_cast<uint64_t*>(smem + 3 * D20H_OP_BYTES);
@@ -270,11 +279,15 @@ edgeconv_dg20_h_kernel(const __grid_constant__ CUtensorMap tmap_w2, Dg20hParams 
     uint64_t* tfull = yempty + 2;
     uint64_t* tempty = tfull + 2;
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
-    constexpr int D20_K = KK, D20_SLOT = DgH<KK>::SLOT, D20_PTS = DgH<KK>::PTS, D20_GROUP_WARPS = DgH<KK>::GROUP_WARPS, D20_THREADS = DgH<KK>::THREADS, ROWQ = DgH<KK>::ROWQ;
+    constexpr int D20_K = KK, D20_SLOT = DgH<KK, C>::SLOT, D20_PTS = DgH<KK, C>::PTS, D20_GROUP_WARPS = DgH<KK, C>::GROUP_WARPS, D20_THREADS = DgH<KK, C>::THREADS, ROWQ = DgH<KK, C>::ROWQ;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
     for (uint32_t i = threadIdx.x; i < 2 * D20H_OP_BYTES / 16; i += D20_THREADS)
         reinterpret_cast<uint4*>(y_s)[i] = make_uint4(0, 0, 0, 0);
+    if constexpr (C < 128) {                           // rows C..127 of the A tile (W2 padded to M = 128) are never loaded
+        for (uint32_t i = threadIdx.x; i < (128 - C) * 128 / 16; i += D20_THREADS)
+            reinterpret_cast<uint4*>(w_s + C * 128)[i] = make_uint4(0, 0, 0, 0);
+    }
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     if (warp == D20_ALLOC_WARP) {
         if (lane == 0) {
@@ -284,7 +297,7 @@ edgeconv_dg20_h_kernel(const __grid_constant__ CUtensorMap tmap_w2, Dg20hParams 
                 mbar_init(&yfull[s], D20_GROUP_WARPS);
                 mbar_init(&yempty[s], 1);
                 mbar_init(&tfull[s], 1);
-                mbar_init(&tempty[s], D20_EPI_WARPS);
+                mbar_init(&tempty[s], EPI_LIVE);
             }
             asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
         }
@@ -300,11 +313,11 @@ edgeconv_dg20_h_kernel(const __grid_constant__ CUtensorMap tmap_w2, Dg20hParams 
     if (warp >= D20_EPI_WARPS) {
         const int pwarp = warp - D20_EPI_WARPS;
         const int grp = pwarp / D20_GROUP_WARPS, gw = pwarp % D20_GROUP_WARPS;
-        const int pl = gw >> 1, chalf = gw & 1;                    // point slot, 64-channel k-block
+        const int pl = gw >> (KBS - 1), chalf = gw & (KBS - 1);    // point slot, 64-channel k-block
         const bool issuer = gw == 0;
         if (warp == D20_ALLOC_WARP && lane == 0) {
-            mbar_expect_tx(wfull, D20H_OP_BYTES);
-            for (int kb2 = 0; kb2 < 2; ++kb2) tma_load_2d(w_s + kb2 * D20H_KB_BYTES, &tmap_w2, wfull, kb2 * 64, 0);
+            mbar_expect_tx(wfull, C * C * 2);
+            for (int kb2 = 0; kb2 < KBS; ++kb2) tma_load_2d(w_s + kb2 * D20H_KB_BYTES, &tmap_w2, wfull, kb2 * 64, 0);
         }
         // kind::f16, fp16 operands, fp32 accumulate, M = N = 128
         constexpr uint32_t idesc = (1u << 4) | ((uint32_t)(128 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
@@ -395,7 +408,7 @@ edgeconv_dg20_h_kernel(const __grid_constant__ CUtensorMap tmap_w2, Dg20hParams 
                 tc_fence_after();
                 const uint32_t y_addr = smem_u32(y_s + grp * D20H_OP_BYTES);
 #pragma unroll
-                for (int kb2 = 0; kb2 < 2; ++kb2) {
+                for (int kb2 = 0; kb2 < KBS; ++kb2) {
                     const uint64_t da = make_smem_desc(w_addr + kb2 * D20H_KB_BYTES), db = make_smem_desc(y_addr + kb2 * D20H_KB_BYTES);
 #pragma unroll
                     for (int ks = 0; ks < 4; ++ks) {             // 16 channels = 32 bytes per MMA
@@ -414,7 +427,7 @@ edgeconv_dg20_h_kernel(const __grid_constant__ CUtensorMap tmap_w2, Dg20hParams 
             }
             __syncwarp();
         }
-    } else {
+    } else if (warp < EPI_LIVE) {
         const int ch = warp * 32 + lane;
         const float s2 = __ldg(P.s2 + ch), t2 = __ldg(P.t2 + ch);
         long long t = blockIdx.x;
@@ -520,16 +533,26 @@ int dg20_tc_run(const float* p, int ldp, const float* q, int ldq, const int32_t*
     return LPD_OK;
 }
 
+template <int KK, int C>
+static int dgh_launch(const Dg20hParams& P, const CUtensorMap& tw, int grid, cudaStream_t st) {
+    constexpr size_t smem = 3 * (size_t)DgH<KK, C>::OP_BYTES + 256;
+    LPD_CUDA_CHECK(allow_smem(edgeconv_dg20_h_kernel<KK, C>, smem));
+    edgeconv_dg20_h_kernel<KK, C><<<grid, DgH<KK, C>::THREADS, smem, st>>>(tw, P);
+    LPD_LAUNCH_CHECK();
+    return LPD_OK;
+}
+
 }  // namespace tc
 }  // namespace lpd
 
-static int edgeconv_dgk_f16(const void* p, int ldp, const void* q, int ldq, const int32_t* idx, int B, int N, int K,
+// C = 128 or 64 channels (p, q, W2 [C][C], x1, x2)
+static int edgeconv_dgk_f16(const void* p, int ldp, const void* q, int ldq, const int32_t* idx, int B, int N, int K, int C,
                             const void* w2, const float* s2, const float* t2, int act, float slope,
                             void* x1, int ld1, void* x2, int ld2, void* stream) {
     using namespace lpd;
     LPD_REQUIRE(p && q && idx && w2 && s2 && t2 && x2 && B >= 1 && (K == 20 || K == 32) && N >= K);
     LPD_REQUIRE(ldp % 8 == 0 && ldq % 8 == 0 && ld2 % 2 == 0 && (!x1 || ld1 % 8 == 0));
-    LPD_REQUIRE(ldp >= 128 && ldq >= 128 && ld2 >= 128 && (!x1 || ld1 >= 128));
+    LPD_REQUIRE(ldp >= C && ldq >= C && ld2 >= C && (!x1 || ld1 >= C));
     LPD_REQUIRE((long long)N * ldp < (1ll << 31));
     LPD_REQUIRE(((uintptr_t)p & 15) == 0 && ((uintptr_t)q & 15) == 0 && ((uintptr_t)x1 & 15) == 0 && ((uintptr_t)x2 & 3) == 0 && ((uintptr_t)w2 & 15) == 0);
     LPD_REQUIRE(act_is_slope(act, slope));
@@ -543,32 +566,31 @@ static int edgeconv_dgk_f16(const void* p, int ldp, const void* q, int ldq, cons
     P.x1 = reinterpret_cast<__half*>(x1); P.x2 = reinterpret_cast<__half*>(x2);
     P.ldp = ldp; P.ldq = ldq; P.ld1 = ld1; P.ld2 = ld2; P.total_pts = (long long)B * N; P.N = N;
     P.neg_slope = act_neg_slope(act, slope);
-    const int pts = K == 32 ? tc::DgH<32>::PTS : tc::DgH<20>::PTS;
+    const int pts = K == 32 ? tc::DgH<32, 128>::PTS : tc::DgH<20, 128>::PTS;
     P.num_tiles = (P.total_pts + pts - 1) / pts;
-    CUtensorMap tw;   // W2 fp16 [128][128]: boxes of 128 rows x 64 halves
-    rc = tc::make_tmap(&tw, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, w2, 128, 128, 128, 128, 64);
+    CUtensorMap tw;   // W2 fp16 [C][C]: boxes of C rows x 64 halves
+    rc = tc::make_tmap(&tw, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, w2, C, C, C, C, 64);
     if (rc != LPD_OK) return rc;
-    constexpr size_t smem = 3 * (size_t)tc::D20H_OP_BYTES + 256;
     const int grid = (int)(P.num_tiles < sms ? P.num_tiles : sms);
-    if (K == 32) {
-        LPD_CUDA_CHECK(allow_smem(tc::edgeconv_dg20_h_kernel<32>, smem));
-        tc::edgeconv_dg20_h_kernel<32><<<grid, tc::DgH<32>::THREADS, smem, as_stream(stream)>>>(tw, P);
-    } else {
-        LPD_CUDA_CHECK(allow_smem(tc::edgeconv_dg20_h_kernel<20>, smem));
-        tc::edgeconv_dg20_h_kernel<20><<<grid, tc::DgH<20>::THREADS, smem, as_stream(stream)>>>(tw, P);
-    }
-    LPD_LAUNCH_CHECK();
-    return LPD_OK;
+    cudaStream_t st = as_stream(stream);
+    if (C == 128) return K == 32 ? tc::dgh_launch<32, 128>(P, tw, grid, st) : tc::dgh_launch<20, 128>(P, tw, grid, st);
+    return K == 32 ? tc::dgh_launch<32, 64>(P, tw, grid, st) : tc::dgh_launch<20, 64>(P, tw, grid, st);
 }
 
 extern "C" int lpd_edgeconv_dg20_f16(const void* p, int ldp, const void* q, int ldq, const int32_t* idx, int B, int N,
                                      const void* w2, const float* s2, const float* t2, int act, float slope,
                                      void* x1, int ld1, void* x2, int ld2, void* stream) {
-    return edgeconv_dgk_f16(p, ldp, q, ldq, idx, B, N, 20, w2, s2, t2, act, slope, x1, ld1, x2, ld2, stream);
+    return edgeconv_dgk_f16(p, ldp, q, ldq, idx, B, N, 20, 128, w2, s2, t2, act, slope, x1, ld1, x2, ld2, stream);
 }
 
 extern "C" int lpd_edgeconv_dg32_f16(const void* p, int ldp, const void* q, int ldq, const int32_t* idx, int B, int N,
                                      const void* w2, const float* s2, const float* t2, int act, float slope,
                                      void* x1, int ld1, void* x2, int ld2, void* stream) {
-    return edgeconv_dgk_f16(p, ldp, q, ldq, idx, B, N, 32, w2, s2, t2, act, slope, x1, ld1, x2, ld2, stream);
+    return edgeconv_dgk_f16(p, ldp, q, ldq, idx, B, N, 32, 128, w2, s2, t2, act, slope, x1, ld1, x2, ld2, stream);
+}
+
+extern "C" int lpd_edgeconv_dg64_f16(const void* p, int ldp, const void* q, int ldq, const int32_t* idx, int B, int N, int k,
+                                     const void* w2, const float* s2, const float* t2, int act, float slope,
+                                     void* x2, int ld2, void* stream) {
+    return edgeconv_dgk_f16(p, ldp, q, ldq, idx, B, N, k, 64, w2, s2, t2, act, slope, nullptr, 0, x2, ld2, stream);
 }

@@ -218,10 +218,10 @@ def gemm(A, B, *, a_layout=A_MK, b_layout=B_NK, M, N, K, lda=None, ldb=None, out
 # ---- precision mode of the dense conv / linear layers ----------------------------------------------------------
 #   "fp32": every GEMM on the CUDA cores (lpd_gemm, plain FFMA)        — strict parity mode
 #   "tf32": large K-contiguous GEMMs on the tensor cores (lpd_gemm_tf32) — fast mode, fp32 operands truncated to TF32 by the MMA
-#   "f16":  the eval path of the reference's own configuration (featnet=lpdnet, k = 20) keeps its activations downstream of the
-#           feature-space kNN in FP16 (rounded to nearest, 11 significant bits) and multiplies on tcgen05 kind::f16 with fp32
-#           accumulation: half the bytes, twice the tensor rate, and a SMALLER error than "tf32" (measured 1e-5 vs 5e-5 max-abs on
-#           the reference goldens).  Everything else (training, the other feature nets) behaves as in "tf32".
+#   "f16":  the eval path of the LPD-Net feature nets (featnet=lpdnet and lpdnetorigin, k = 20 or 32) keeps its activations
+#           downstream of the feature-space kNN in FP16 (rounded to nearest, 11 significant bits) and multiplies on tcgen05 kind::f16
+#           with fp32 accumulation: half the bytes, twice the tensor rate, and a SMALLER error than "tf32" (measured 1e-5 vs 5e-5
+#           max-abs on the reference goldens).  Everything else (training, featnet=pointnet, other k) behaves as in "tf32".
 _precision = "fp32"
 
 
@@ -359,7 +359,7 @@ def softmax64_f16(a, M):
 
 
 def edge_gather_max_f16(p, ldp, q, ldq, idx, B, N, k, C, act, slope, out, ldo):
-    """out = act(q + max_m p[j(i,m)]) on fp16 rows (C == 256): lpd_edge_gather_max_f16"""
+    """out = act(q + max_m p[j(i,m)]) on fp16 rows (C == 256 or 64): lpd_edge_gather_max_f16"""
     lib = _lib.load()
     _f16(p, "p")
     _call(f"lpd_edge_gather_ext[C={C}]", 1, lib.lpd_edge_gather_max_f16, p.data_ptr(), ldp, _p(q), ldq, idx.data_ptr(), B, N, k, C,
@@ -378,6 +378,17 @@ def edgeconv_dg20_f16(p, ldp, q, ldq, idx, B, N, w2_h, s2, t2, act, slope, x1, l
     _call("lpd_edgeconv_dg_f16[128x128]", 1, lib.lpd_edgeconv_dg20_f16 if k == 20 else lib.lpd_edgeconv_dg32_f16, p.data_ptr(), ldp, q.data_ptr(), ldq, idx.data_ptr(), B, N,
           w2_h.data_ptr(), s2.data_ptr(), t2.data_ptr(), act, float(slope), _p(x1), ld1, x2.data_ptr(), ld2, _stream())
     return x1, x2
+
+
+def edgeconv_dg64_f16(p, ldp, q, ldq, idx, B, N, w2_h, s2, t2, act, slope, x2, ld2):
+    """LPDNetOrign's 64-channel double edge layer with fp16 rows in and out (lpd_edgeconv_dg64_f16); k = idx.shape[-1], and any
+    k but 20 or 32 is rejected by the library"""
+    lib = _lib.load()
+    _f16(p, "p"), _f16(q, "q"), _f16(w2_h, "w2"), _f16(x2, "x2")
+    k = idx.shape[-1]
+    _call("lpd_edgeconv_dg_f16[64x64]", 1, lib.lpd_edgeconv_dg64_f16, p.data_ptr(), ldp, q.data_ptr(), ldq, idx.data_ptr(), B, N,
+          k, w2_h.data_ptr(), s2.data_ptr(), t2.data_ptr(), act, float(slope), x2.data_ptr(), ld2, _stream())
+    return x2
 
 
 def _tn_ok(A, Bm, M, N, K, lda, ldb, batch):

@@ -348,7 +348,7 @@ class PointNetVlad(nn.Module):
             return forward_train(self, x)
         if self.emb_nn is not None:
             # "f16" precision mode: fp16 activations downstream of the kNN, for the configuration the kernels are specialised for
-            f16 = (ops.get_precision() == "f16" and isinstance(self.emb_nn, LPDNet) and self.emb_nn.k in (20, 32) and x.size(2) % 64 == 0
+            f16 = (ops.get_precision() == "f16" and isinstance(self.emb_nn, (LPDNet, LPDNetOrign)) and self.emb_nn.k in (20, 32) and x.size(2) % 64 == 0
                    and x.size(0) * x.size(2) >= 128 and self.net_vlad.cluster_size == 64 and self.net_vlad.feature_size % 8 == 0)
             f, B, N = self.emb_nn.forward_pm(x, f16=True) if f16 else self.emb_nn.forward_pm(x)
         else:

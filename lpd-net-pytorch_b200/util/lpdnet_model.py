@@ -337,9 +337,18 @@ class LPDNetOrign(_LPDBase):
         p["wsn1"], p["wsn2"] = w2d(self.convSN1[0].weight), w2d(self.convSN2[0].weight)
         p["ssn1"], p["tsn1"] = fold_bn(self.convSN1[1])
         p["ssn2"], p["tsn2"] = fold_bn(self.convSN2[1])
+        # epilogue vectors of the DG1 projection for the pre-scaled f16 edge kernel: P' = s1 P, Q' = s1 Q + t1
+        p["spq1"] = torch.cat((p["sdg1"], p["sdg1"])).contiguous()
+        p["tpq1"] = torch.cat((torch.zeros_like(p["tdg1"]), p["tdg1"])).contiguous()
+        if p["w3"].is_cuda:      # fp16 copies of the weights the "f16" precision mode multiplies with (rounded to nearest, once)
+            for name in ("wdg2", "wsn1", "wsn2", "w3", "w4", "w5"):
+                p[name + "_h"] = ops.to_f16(p[name])
         return p
 
-    def forward_pm(self, x: torch.Tensor, keep_order: bool = False):
+    def forward_pm(self, x: torch.Tensor, keep_order: bool = False, f16: bool = False):
+        """-> (F [B*N, emb] point-major, B, N), rows in spatial order unless keep_order (see LPDNet.forward_pm).
+        f16 (PointNetVlad.forward in "f16" precision mode, k == 20 or 32): F and every activation downstream of the feature-space kNN
+        are fp16 tensors; conv1 / conv2 and both kNN graphs stay exact fp32."""
         require_cuda(x, "LPDNetOrign")
         training_unsupported(self, "LPDNetOrign")
         p = self._prep.get(self, self._build)
@@ -348,6 +357,20 @@ class LPDNetOrign(_LPDBase):
         act, slope = _act_code(self)
         dev = h.device
         idx_f = ops.knn(h.view(B, N, 64), k)
+        if f16 and k in (20, 32) and M >= 128 and self.emb_dims % 8 == 0:
+            pq1 = ops.gemm_tf32_out16(h, p["wpq1"], M=M, N=128, K=64, scale=p["spq1"], shift=p["tpq1"])
+            xdg = torch.empty(M, 64, device=dev, dtype=torch.float16)
+            ops.edgeconv_dg64_f16(pq1, 128, pq1[:, 64:], 128, idx_f, B, N, p["wdg2_h"], p["sdg2"], p["tdg2"], act, slope, xdg, 64)
+            del pq1
+            idx_x = ops.knn(xyz_init, k)
+            g = ops.gemm_f16(xdg, p["wsn1_h"], M=M, N=64, K=64, out_half=True, scale=p["ssn1"], shift=p["tsn1"], act=act, slope=slope)
+            g = ops.gemm_f16(g, p["wsn2_h"], M=M, N=64, K=64, out_half=True, scale=p["ssn2"], shift=p["tsn2"], act=act, slope=slope)
+            xsn = torch.empty(M, 64, device=dev, dtype=torch.float16)
+            ops.edge_gather_max_f16(g, 64, None, 0, idx_x, B, N, k, 64, ops.ACT_NONE, 0.0, xsn, 64)
+            f = ops.gemm_f16(xsn, p["w3_h"], M=M, N=64, K=64, out_half=True, scale=p["s3"], shift=p["t3"], act=act, slope=slope)
+            f = ops.gemm_f16(f, p["w4_h"], M=M, N=128, K=64, out_half=True, scale=p["s4"], shift=p["t4"], act=act, slope=slope)
+            f = ops.gemm_f16(f, p["w5_h"], M=M, N=self.emb_dims, K=128, out_half=True, scale=p["s5"], shift=p["t5"], act=act, slope=slope)
+            return f, B, N
         pq1 = ops.linear(h, p["wpq1"], M=M, N=128, K=64)
         xdg = torch.empty(M, 64, device=dev, dtype=torch.float32)
         ops.edgeconv_dg(pq1, 128, pq1[:, 64:], 128, idx_f, B, N, k, 64, 64, p["sdg1"], p["tdg1"], p["wdg2"],
