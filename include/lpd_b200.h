@@ -189,6 +189,16 @@ int lpd_gemm_f16(const void* A, int lda, const void* W, int ldw, void* C, int ld
 int lpd_gemm_f16_tn(const void* A, int lda, const void* B, int ldb, float* C, int ldc, long long strideC,
                     int M, int N, int K, int batch, void* stream);
 int lpd_f32_to_f16(const float* x, long long ldx, void* y, long long ldy, long long rows, int cols, void* stream);
+/* lpd_gemm_f16 followed by a max over each cloud's R rows, without writing the [M][N] product (PointNetVlad.py:164-169, the STN's
+ * conv3 + bn3 + relu + mp1):
+ *     out[b][n] = max_{r < R} act(scale[n] * sum_k A[b*R + r][k] W[n][k] + shift[n])        out fp32 [M/R][N]
+ * A [M][lda], W [N][ldw] fp16; scale / shift may be NULL.  The GEMM epilogue writes the column maxima of every 32-row block to
+ * part (fp32 [M/32][N], caller-provided, no initialisation needed), and lpd_colmax reduces those per cloud in the same call.
+ * Each element goes through the same epilogue as lpd_gemm_f16 with fp32 output, so out equals lpd_colmax of that product exactly.
+ * Requires R % 32 == 0, M % R == 0, M / R <= 65535, N % 256 == 0, lda, ldw % 8 == 0, 16-byte aligned pointers and act in
+ * {NONE, RELU, LEAKY with 0 <= slope <= 1}; otherwise LPD_EINVAL with nothing launched. */
+int lpd_gemm_f16_colmax(const void* A, int lda, const void* W, int ldw, int M, int N, int K, int R,
+                        const float* scale, const float* shift, int act, float slope, float* part, float* out, void* stream);
 /* "3xTF32" operand preparation: x (n contiguous floats) = hi + lo, hi = x truncated to TF32, lo = x - hi; out [3][n] holds
  * [hi; hi; lo] (role 0, the A side) or [hi; lo; hi] (role 1, the B side), so that one lpd_gemm_tf32_tn contraction over the stacked
  * rows accumulates hi.hi + hi.lo + lo.hi in fp32.  Used by the NetVLAD hidden projection (65536 x 256, PointNetVlad.py:76), which

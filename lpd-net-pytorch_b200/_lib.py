@@ -46,6 +46,7 @@ SIGNATURES = {
     "lpd_gemm_tf32_tn": (_i, [_vp, _i, _vp, _i, _vp, _i, _ll, _i, _i, _i, _i, _vp]),
     "lpd_gemm_f16": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _f, _vp]),
     "lpd_gemm_f16_tn": (_i, [_vp, _i, _vp, _i, _vp, _i, _ll, _i, _i, _i, _i, _vp]),
+    "lpd_gemm_f16_colmax": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _i, _f, _vp, _vp, _vp]),
     "lpd_f32_to_f16": (_i, [_vp, _ll, _vp, _ll, _ll, _i, _vp]),
     "lpd_split3_tf32": (_i, [_vp, _ll, _vp, _i, _vp]),
     "lpd_transpose_split3": (_i, [_vp, _i, _ll, _i, _vp, _vp]),

@@ -19,6 +19,10 @@
 // 128-byte shared-memory row, K = 16 per MMA — the byte geometry of the pipeline is unchanged — and can write its output as
 // fp16 (OUT_HALF).  That is the "f16" precision mode of the eval path: operands rounded to nearest fp16 (11 significant
 // bits, vs the 10-bit TRUNCATION kind::tf32 applies to fp32 operands), twice the tensor rate and half the operand bytes.
+//
+// Epilogue forms (template parameter EPI): 0 stores the affine + activation result; 1 (BN = 64) a row softmax (NetVLAD soft
+// assignment); 2 (fp16 operands, BN = 256) stores only the column maxima of every 32-row block, for a GEMM followed by a max
+// over each cloud's points (lpd_gemm_f16_colmax).
 #include "tc_common.cuh"
 #include <cuda_fp16.h>
 
@@ -41,6 +45,7 @@ struct Params {
     int accumulate = 0;             // !TN: C += result (the epilogue reads C)
     // EPI == 1 (BN == 64): row softmax of the affine result instead of the activation; C (fp32, may be null), a_h (fp16 copy, may
     // be null) and apart[row block of 32][64] = the column sums of every 32-row block (may be null)
+    // EPI == 2 (BN == 256, M % 32 == 0): C is not written; apart[row block of 32][N] = the column maxima of every 32-row block
     __half* a_h = nullptr; float* apart = nullptr;
 };
 
@@ -92,7 +97,8 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
     uint64_t* tempty = tfull + 2;
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 2);
     float* xch = reinterpret_cast<float*>(tmem_slot + 2);       // EPI == 1: [2][4 quarters][2 halves][32 rows] row max / row sum
-    static_assert(EPI == 0 || (BN == 64 && !TN && !OUT_HALF), "the softmax epilogue covers one 64-column tile");
+    static_assert(EPI != 1 || (BN == 64 && !TN && !OUT_HALF), "the softmax epilogue covers one 64-column tile");
+    static_assert(EPI != 2 || (BN == 256 && !TN && !OUT_HALF && HALF), "the column-max epilogue is the fp16 256-column form");
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int num_kb = (p.K + BKE - 1) / BKE;
@@ -253,12 +259,14 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
             for (int i = 0; i < CPW; ++i) {
                 const int c = half * CPW + i;
                 const int col0 = n0 + c * 32;
-                if (col0 >= p.N || row0 >= p.M) break;  // warp-uniform: the rest is out of range
+                // warp-uniform: the rest is out of range.  EPI == 2 relies on it: with M % 32 == 0 a lane quarter is all rows < M
+                // or all rows >= M, and the TMA zero-filled rows (act(shift) after the epilogue) must not enter a maximum.
+                if (col0 >= p.N || row0 >= p.M) break;
                 // accumulate mode: the old C values of this lane's 8 rows are requested before the accumulators are read, so
                 // their latency overlaps the TMEM load and the staging pass instead of sitting in the store loop
                 const int colp = col0 + ch * 4;
                 float4 oldc[8];
-                if (!TN && p.accumulate) {
+                if (EPI == 0 && !TN && p.accumulate) {
                     const float* gold = p.C + (size_t)z * p.bM * p.ldc + (size_t)row0 * p.ldc + colp;
 #pragma unroll
                     for (int it = 0; it < 8; ++it) {
@@ -284,6 +292,7 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                 const size_t goff = (TN ? (size_t)z * p.strideC : (size_t)z * p.bM * p.ldc) + (size_t)row0 * p.ldc + col;
                 float* gcol = p.C + goff;
                 __half* hcol = reinterpret_cast<__half*>(p.C) + goff;          // OUT_HALF: C is an fp16 matrix (ldc in halves)
+                float4 mx = make_float4(-INFINITY, -INFINITY, -INFINITY, -INFINITY);   // EPI == 2: max over this lane's 8 rows
 #pragma unroll
                 for (int it = 0; it < 8; ++it) {
                     const int rr = it * 4 + rsub;
@@ -291,7 +300,9 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                     v.x = fmaf(v.x, sc.x, sh.x); v.y = fmaf(v.y, sc.y, sh.y); v.z = fmaf(v.z, sc.z, sh.z); v.w = fmaf(v.w, sc.w, sh.w);
                     v.x = fmaxf(v.x, v.x * p.neg_slope); v.y = fmaxf(v.y, v.y * p.neg_slope);
                     v.z = fmaxf(v.z, v.z * p.neg_slope); v.w = fmaxf(v.w, v.w * p.neg_slope);
-                    if (col_ok && row0 + rr < p.M) {
+                    if constexpr (EPI == 2) {
+                        mx.x = fmaxf(mx.x, v.x); mx.y = fmaxf(mx.y, v.y); mx.z = fmaxf(mx.z, v.z); mx.w = fmaxf(mx.w, v.w);
+                    } else if (col_ok && row0 + rr < p.M) {
                         if (OUT_HALF) {
                             __half2 h0, h1;                                      // saturating: out-of-range values become +-65504, not inf
                             asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(*reinterpret_cast<uint32_t*>(&h0)) : "f"(v.y), "f"(v.x));
@@ -304,6 +315,16 @@ gemm_tf32_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                             *dstp = v;
                         }
                     }
+                }
+                if constexpr (EPI == 2) {
+                    // lanes ch, ch + 8, ch + 16, ch + 24 hold the same 4 columns for rows rsub, rsub + 4, ...: combine the four
+                    // row groups, then one 16-byte store per column group gives the block's row of apart
+#pragma unroll
+                    for (int o = 8; o <= 16; o <<= 1) {
+                        mx.x = fmaxf(mx.x, __shfl_xor_sync(kFull, mx.x, o)); mx.y = fmaxf(mx.y, __shfl_xor_sync(kFull, mx.y, o));
+                        mx.z = fmaxf(mx.z, __shfl_xor_sync(kFull, mx.z, o)); mx.w = fmaxf(mx.w, __shfl_xor_sync(kFull, mx.w, o));
+                    }
+                    if (lane < 8) *reinterpret_cast<float4*>(p.apart + (size_t)(row0 >> 5) * p.N + col) = mx;
                 }
                 __syncwarp();                            // staging buffer is rewritten by the next chunk
             }
@@ -601,6 +622,7 @@ struct GemmCall {
     bool tn = false;
     bool out_half = false;   // C is fp16
     bool softmax = false;    // EPI 1: row softmax over N == 64 columns
+    bool colmax = false;     // EPI 2: fp16 operands, N % 256 == 0, column maxima of every 32-row block into p.apart
     Params p;
 };
 
@@ -615,6 +637,9 @@ static int launch_bn(int BN, const CUtensorMap& ta, const CUtensorMap& tb, const
 template <typename TIN>
 static int launch_form(const GemmCall& g, int BN, const CUtensorMap& ta, const CUtensorMap& tb, cudaStream_t st) {
     if (g.softmax) return launch<64, 8, false, TIN, false, 1>(ta, tb, g.p, st);
+    if constexpr (sizeof(TIN) == 2) {
+        if (g.colmax) return launch<256, 4, false, TIN, false, 2>(ta, tb, g.p, st);
+    }
     if (g.tn) return launch_bn<TIN, true, false>(BN, ta, tb, g.p, st);
     if (g.out_half) return launch_bn<TIN, false, true>(BN, ta, tb, g.p, st);
     return launch_bn<TIN, false, false>(BN, ta, tb, g.p, st);
@@ -626,7 +651,7 @@ static int gemm_run(const GemmCall& g, cudaStream_t st) {
     const Params& p = g.p;
     // CTA-pair kernel: wide layers whose epilogue scale / shift fit its shared memory, with fp16 output (16-byte row stores) or
     // as one large fp32 product
-    const bool pair = !g.tn && !g.softmax && (p.N % 256) == 0 && p.N <= H2_MAXN &&
+    const bool pair = !g.tn && !g.softmax && !g.colmax && (p.N % 256) == 0 && p.N <= H2_MAXN &&
                       (g.out_half ? (p.ldc % 8) == 0 : !g.half && p.batch == 1 && !p.accumulate && p.M >= 1024);
     const int BN = p.N <= 64 ? 64 : (p.N <= 128 ? 128 : 256);
     const CUtensorMapDataType type = g.half ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
@@ -752,6 +777,25 @@ extern "C" int lpd_gemm_f16(const void* A, int lda, const void* W, int ldw, void
     g.p.C = reinterpret_cast<float*>(C); g.p.ldc = ldc; g.p.M = M; g.p.N = N; g.p.K = K; g.p.scale = scale; g.p.shift = shift;
     g.p.neg_slope = act_neg_slope(act, slope);
     return tc::gemm_run(g, as_stream(stream));
+}
+
+extern "C" int lpd_gemm_f16_colmax(const void* A, int lda, const void* W, int ldw, int M, int N, int K, int R,
+                                   const float* scale, const float* shift, int act, float slope, float* part, float* out,
+                                   void* stream) {
+    using namespace lpd;
+    LPD_REQUIRE(A && W && part && out && M >= 1 && N >= 1 && K >= 1 && R >= 1);
+    LPD_REQUIRE(lda >= K && ldw >= K && (lda % 8) == 0 && (ldw % 8) == 0);
+    LPD_REQUIRE((R % 32) == 0 && (M % R) == 0 && (N % 256) == 0 && M / R <= 65535);
+    LPD_REQUIRE(((uintptr_t)A & 15) == 0 && ((uintptr_t)W & 15) == 0 && ((uintptr_t)part & 15) == 0 && ((uintptr_t)out & 15) == 0 &&
+                ((uintptr_t)scale & 15) == 0 && ((uintptr_t)shift & 15) == 0);
+    LPD_REQUIRE(act_is_slope(act, slope));
+    tc::GemmCall g;
+    g.A = A; g.lda = lda; g.B = W; g.ldb = ldw; g.half = true; g.colmax = true;
+    g.p.M = M; g.p.N = N; g.p.K = K; g.p.scale = scale; g.p.shift = shift; g.p.apart = part;
+    g.p.neg_slope = act_neg_slope(act, slope);
+    const int rc = tc::gemm_run(g, as_stream(stream));
+    if (rc != LPD_OK) return rc;
+    return lpd_colmax(part, M / R, R / 32, N, N, out, stream);       // each cloud's R / 32 block maxima
 }
 
 extern "C" int lpd_gemm_f16_tn(const void* A, int lda, const void* B, int ldb, float* C, int ldc, long long strideC,

@@ -218,10 +218,12 @@ def gemm(A, B, *, a_layout=A_MK, b_layout=B_NK, M, N, K, lda=None, ldb=None, out
 # ---- precision mode of the dense conv / linear layers ----------------------------------------------------------
 #   "fp32": every GEMM on the CUDA cores (lpd_gemm, plain FFMA)        — strict parity mode
 #   "tf32": large K-contiguous GEMMs on the tensor cores (lpd_gemm_tf32) — fast mode, fp32 operands truncated to TF32 by the MMA
-#   "f16":  the eval path of the LPD-Net feature nets (featnet=lpdnet and lpdnetorigin, k = 20 or 32) keeps its activations
-#           downstream of the feature-space kNN in FP16 (rounded to nearest, 11 significant bits) and multiplies on tcgen05 kind::f16
-#           with fp32 accumulation: half the bytes, twice the tensor rate, and a SMALLER error than "tf32" (measured 1e-5 vs 5e-5
-#           max-abs on the reference goldens).  Everything else (training, featnet=pointnet, other k) behaves as in "tf32".
+#   "f16":  the eval path of all three feature nets (featnet=lpdnet and lpdnetorigin at k = 20 or 32: downstream of the
+#           feature-space kNN; featnet=pointnet at N % 64 == 0: after conv2, and the STNs' conv2 / conv3) keeps its activations in
+#           FP16 (rounded to nearest, 11 significant bits) and multiplies on tcgen05 kind::f16 with fp32 accumulation: half the
+#           bytes, twice the tensor rate, and a SMALLER error than "tf32" (measured 1e-5 vs 5e-5 max-abs on the lpdnet golden,
+#           2e-5 / 4.5e-5 vs 7e-5 / 1.3e-4 on the two pointnet goldens).  Everything else (training, other k, other N) behaves as
+#           in "tf32".
 _precision = "fp32"
 
 
@@ -326,6 +328,19 @@ def gemm_f16(A, W, *, M, N, K, lda=None, ldw=None, out=None, ldc=None, out_half=
             ldc = out.stride(-2)
     _call(f"lpd_gemm_f16[{M}x{N}x{K}]", 1, lib.lpd_gemm_f16, A.data_ptr(), lda, W.data_ptr(), ldw, out.data_ptr(), ldc, int(out_half),
           M, N, K, _p(scale), _p(shift), act, float(slope), _stream())
+    return out
+
+
+def gemm_f16_colmax(A, W, *, M, N, K, R, scale=None, shift=None, act, slope):
+    """out[b][n] = max_{r<R} act(scale[n] * sum_k A[b*R + r][k] W[n][k] + shift[n]) -> fp32 [M/R, N], fp16 operands on the tensor
+    cores; the [M, N] product is never written (lpd_gemm_f16_colmax: R % 32 == 0, N % 256 == 0).  Allocates, besides the output,
+    an fp32 [M/32, N] scratch buffer for the column maxima of every 32-row block."""
+    lib = _lib.load()
+    _f16(A, "A"), _f16(W, "W")
+    part = torch.empty(M // 32, N, device=A.device, dtype=torch.float32)
+    out = torch.empty(M // R, N, device=A.device, dtype=torch.float32)
+    _call(f"lpd_gemm_f16_colmax[{M}x{N}x{K}]", 2, lib.lpd_gemm_f16_colmax, A.data_ptr(), A.stride(0), W.data_ptr(), W.stride(0), M, N, K,
+          R, _p(scale), _p(shift), act, float(slope), part.data_ptr(), out.data_ptr(), _stream())
     return out
 
 

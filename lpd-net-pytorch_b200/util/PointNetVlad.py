@@ -216,10 +216,17 @@ class STN3d(nn.Module):
                 p[f"s{i}"], p[f"t{i}"] = None, lin.bias.detach()
         p["w6"] = w2d(self.fc3.weight)
         p["t6"] = self.fc3.bias.detach() + torch.eye(self.k, device=self.fc3.bias.device).reshape(-1)
+        if p["w3"].is_cuda:      # fp16 copies of the weights the "f16" precision mode multiplies with (rounded to nearest, once)
+            p["w3_h"] = ops.to_f16(p["w3"])
+            if self.k == 64:
+                p["w2_h"] = ops.to_f16(p["w2"])
         return p
 
-    def forward_pm(self, rows: torch.Tensor, B: int, N: int) -> torch.Tensor:
-        """rows [B*N, k] point-major -> [B, k, k]"""
+    def forward_pm(self, rows: torch.Tensor, B: int, N: int, f16: bool = False) -> torch.Tensor:
+        """rows [B*N, k] point-major -> [B, k, k].
+        f16 (PointNetfeat.forward_pm in "f16" precision mode; needs N % 32 == 0): the per-point activations that feed conv3 (and conv2 for
+        k == 64) are fp16 tensors, and conv3 + ReLU + max over the points run in one call without writing the [B*N, 1024] map;
+        fc1-fc3 stay fp32."""
         if self.use_bn:
             training_unsupported(self, "STN3d")
         if N != self.num_points:
@@ -227,10 +234,19 @@ class STN3d(nn.Module):
                              f"(the reference's MaxPool2d((num_points,1)) silently mis-pools here)")
         p = self._prep.get(self, self._build)
         M, R = B * N, ops.ACT_RELU
-        h = ops.linear(rows, p["w1"], M=M, N=64, K=self.k, scale=p["s1"], shift=p["t1"], act=R)
-        h = ops.linear(h, p["w2"], M=M, N=128, K=64, scale=p["s2"], shift=p["t2"], act=R)
-        h = ops.linear(h, p["w3"], M=M, N=1024, K=128, scale=p["s3"], shift=p["t3"], act=R)
-        g = ops.colmax(h, B, N, 1024)
+        if f16:
+            if self.k == 3:     # K = 3: fp32 CUDA-core layer, fp32 operands of conv2 consumed as TF32
+                h = ops.linear(rows, p["w1"], M=M, N=64, K=3, scale=p["s1"], shift=p["t1"], act=R)
+                h = ops.gemm_tf32_out16(h, p["w2"], M=M, N=128, K=64, scale=p["s2"], shift=p["t2"], act=R)
+            else:
+                h = ops.gemm_tf32_out16(rows, p["w1"], M=M, N=64, K=self.k, scale=p["s1"], shift=p["t1"], act=R)
+                h = ops.gemm_f16(h, p["w2_h"], M=M, N=128, K=64, out_half=True, scale=p["s2"], shift=p["t2"], act=R)
+            g = ops.gemm_f16_colmax(h, p["w3_h"], M=M, N=1024, K=128, R=N, scale=p["s3"], shift=p["t3"], act=R, slope=0.0)
+        else:
+            h = ops.linear(rows, p["w1"], M=M, N=64, K=self.k, scale=p["s1"], shift=p["t1"], act=R)
+            h = ops.linear(h, p["w2"], M=M, N=128, K=64, scale=p["s2"], shift=p["t2"], act=R)
+            h = ops.linear(h, p["w3"], M=M, N=1024, K=128, scale=p["s3"], shift=p["t3"], act=R)
+            g = ops.colmax(h, B, N, 1024)
         g = ops.linear(g, p["w4"], M=B, N=512, K=1024, scale=p["s4"], shift=p["t4"], act=R)
         g = ops.linear(g, p["w5"], M=B, N=256, K=512, scale=p["s5"], shift=p["t5"], act=R)
         g = ops.linear(g, p["w6"], M=B, N=self.k * self.k, K=256, shift=p["t6"])
@@ -280,28 +296,40 @@ class PointNetfeat(nn.Module):
             conv, bn = getattr(self, f"conv{i}"), getattr(self, f"bn{i}")
             p[f"w{i}"] = w2d(conv.weight)
             p[f"s{i}"], p[f"t{i}"] = fold_bn(bn, conv.bias)
+        if p["w4"].is_cuda:      # fp16 copies of the weights the "f16" precision mode multiplies with (rounded to nearest, once)
+            p["w4_h"], p["w5_h"] = ops.to_f16(p["w4"]), ops.to_f16(p["w5"])
         return p
 
-    def forward_pm(self, x: torch.Tensor):
-        """x [B,1,N,3] -> (F [B*N, emb] point-major (before any pooling), trans [B,3,3], h2 [B*N,64], B, N)"""
+    def forward_pm(self, x: torch.Tensor, f16: bool = False):
+        """x [B,1,N,3] -> (F [B*N, emb] point-major (before any pooling), trans [B,3,3], h2 [B*N,64], B, N).
+        f16 (PointNetVlad.forward in "f16" precision mode; needs N % 32 == 0): both STNs take their f16 form, conv3-conv5 keep fp16
+        activations and F is an fp16 tensor; the input transform, conv1 / conv2 (h2) and the feature transform stay fp32."""
         require_cuda(x, "PointNetfeat")
         training_unsupported(self, "PointNetfeat")
         p = self._prep.get(self, self._build)
         B, _, N, _ = x.shape
         M, R = B * N, ops.ACT_RELU
         rows = x.detach().reshape(M, 3).contiguous()
-        trans = self.stn.forward_pm(rows, B, N)                                               # :205
+        trans = self.stn.forward_pm(rows, B, N, f16=f16)                                      # :205
         xt = ops.gemm(rows, trans, b_layout=ops.B_KN, M=N, N=3, K=3, lda=3, ldb=3, batch=B,
                       strideA=N * 3, strideB=9, strideC=N * 3,
                       out=torch.empty(M, 3, device=x.device, dtype=torch.float32), ldc=3)     # :209
-        h = ops.linear(xt, p["w1"], M=M, N=64, K=3, scale=p["s1"], shift=p["t1"], act=R)         # :213
-        h2 = ops.linear(h, p["w2"], M=M, N=64, K=64, scale=p["s2"], shift=p["t2"], act=R)        # :215
+        if f16:                                                                               # :213-215 in one strict-fp32 pass
+            h2 = ops.pointwise_mlp2(xt, 3, M, p["w1"], p["s1"], p["t1"], p["w2"], p["s2"], p["t2"], act=R)
+        else:
+            h = ops.linear(xt, p["w1"], M=M, N=64, K=3, scale=p["s1"], shift=p["t1"], act=R)     # :213
+            h2 = ops.linear(h, p["w2"], M=M, N=64, K=64, scale=p["s2"], shift=p["t2"], act=R)    # :215
         h = h2
         if self.apply_feature_trans:                                                          # :218-225
-            ft = self.feature_trans.forward_pm(h2, B, N)
+            ft = self.feature_trans.forward_pm(h2, B, N, f16=f16)
             h = ops.gemm(h2, ft, b_layout=ops.B_KN, M=N, N=64, K=64, lda=64, ldb=64, batch=B,
                          strideA=N * 64, strideB=64 * 64, strideC=N * 64,
                          out=torch.empty(M, 64, device=x.device, dtype=torch.float32), ldc=64)
+        if f16:
+            h = ops.gemm_tf32_out16(h, p["w3"], M=M, N=64, K=64, scale=p["s3"], shift=p["t3"], act=R)                 # :226
+            h = ops.gemm_f16(h, p["w4_h"], M=M, N=128, K=64, out_half=True, scale=p["s4"], shift=p["t4"], act=R)       # :228
+            f = ops.gemm_f16(h, p["w5_h"], M=M, N=self.emb_dims, K=128, out_half=True, scale=p["s5"], shift=p["t5"])   # :230
+            return f, trans, h2, B, N
         h = ops.linear(h, p["w3"], M=M, N=64, K=64, scale=p["s3"], shift=p["t3"], act=R)         # :226
         h = ops.linear(h, p["w4"], M=M, N=128, K=64, scale=p["s4"], shift=p["t4"], act=R)        # :228
         f = ops.linear(h, p["w5"], M=M, N=self.emb_dims, K=128, scale=p["s5"], shift=p["t5"])    # :230 (no ReLU)
@@ -346,15 +374,17 @@ class PointNetVlad(nn.Module):
             # batch-statistics BatchNorm + hand-written backward behind one autograd node (lpdnet_b200/train.py)
             from ..train import forward_train
             return forward_train(self, x)
+        # "f16" precision mode: fp16 activations (downstream of the kNN for the LPD nets), for the configurations the kernels are
+        # specialised for.  N % 64 == 0: the fp16 NetVLAD aggregate contracts each cloud's N rows in 64-row k-blocks.
+        f16 = (ops.get_precision() == "f16" and x.size(2) % 64 == 0 and x.size(0) * x.size(2) >= 128
+               and self.net_vlad.cluster_size == 64 and self.net_vlad.feature_size % 8 == 0)
         if self.emb_nn is not None:
-            # "f16" precision mode: fp16 activations downstream of the kNN, for the configuration the kernels are specialised for
-            f16 = (ops.get_precision() == "f16" and isinstance(self.emb_nn, (LPDNet, LPDNetOrign)) and self.emb_nn.k in (20, 32) and x.size(2) % 64 == 0
-                   and x.size(0) * x.size(2) >= 128 and self.net_vlad.cluster_size == 64 and self.net_vlad.feature_size % 8 == 0)
+            f16 = f16 and isinstance(self.emb_nn, (LPDNet, LPDNetOrign)) and self.emb_nn.k in (20, 32)
             f, B, N = self.emb_nn.forward_pm(x, f16=True) if f16 else self.emb_nn.forward_pm(x)
         else:
             if self.point_net.max_pool:
                 raise ValueError("PointNetVlad needs the per-point feature map: construct with max_pool=False")
-            f, _, _, B, N = self.point_net.forward_pm(x)
+            f, _, _, B, N = self.point_net.forward_pm(x, f16=f16)
         if N != self.net_vlad.max_samples:
             raise ValueError(f"PointNetVlad: got {N} points per cloud, constructed for num_points={self.net_vlad.max_samples}")
         return self.net_vlad.forward_pm(f, B)
