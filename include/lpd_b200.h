@@ -462,6 +462,51 @@ int lpd_edge_bwd_apply(const float* p, int ldp, const float* q, int ldq, const i
                        const float* dy, const float* S, double count, float* dp, int lddp, float* dq, int lddq,
                        void* stream);
 
+/* f16 storage of the edge tensors (the "f16" train precision mode of featnet="lpdnet", set_train_precision in ops.py).
+ * The dense DG2 edge layer keeps its four [M*k][C] tensors in fp16: y1 (input rows), z2e (pre-activations), and their
+ * gradients dz2e and dy1.  Every kernel below computes in fp32 exactly as its fp32 form above does, on the values the fp16
+ * storage holds; fp16 results are rounded to nearest.  Requirements on top of the fp32 forms: C % 8 == 0, 1 <= k <= 255,
+ * fp16 pointers 16-byte aligned, arg 8-byte aligned, non-null scale pointers; otherwise LPD_EINVAL with nothing launched.
+ *   lpd_bn_stats_f16          : lpd_bn_stats over fp16 z (C <= 1024), plus the exact column min / max as order keys in
+ *                               minmax uint32 [2][C] (read by lpd_edge_grad_scale_f16).  |z| >= 65504 (the fp16 limit, where
+ *                               lpd_gemm_f16 saturates) counts as NaN: z must fit fp16's range, or the statistics and with them
+ *                               the loss come out non-finite — never silently wrong.
+ *   lpd_edge_materialize_f16  : lpd_edge_materialize with y stored as fp16 (p, q fp32).
+ *   lpd_edge_sel_dense_f16    : lpd_edge_sel_dense over fp16 z (zsel fp32, arg uint8 as before).
+ *   lpd_edge_dense_bwd_apply_f16: lpd_edge_dense_bwd_apply over fp16 z, writing fp16(2^E * dz) (in place over z allowed).
+ *   lpd_edge_bwd_{reduce,apply}_f16: lpd_edge_bwd_{reduce,apply} with a required fp16 dy holding 2^E * dy; each value is
+ *                               multiplied by dyscale[0] = 2^-E in fp32 (exact) before use.
+ * Gradient scaling.  BN backward over count = M*k edges makes dz2e tiny (below fp16's subnormal floor 6e-8 for many entries
+ * at training sizes), so dz2e and dy1 are stored as fp16(2^E * value) with ONE power-of-two exponent E per step, computed on
+ * the device (no host synchronisation, no skipped steps) from a bound:
+ *     max|dz_c|  <= |scale_c| * (max_i|dx_ic| * max(1, |gneg|) + |S1_c|/count + X_c * |S2_c|/count),
+ *     X_c = max(|min_c - mean_c|, |max_c - mean_c|) * invstd_c   (the column range lpd_bn_stats_f16 recorded),
+ *     max|dy1_k| <= sum_c |W2[c][k]| * max|dz_c|                  (dy1 = dz2e . W2, W2 [C][K] fp16, ldw),
+ * and E is the largest integer with 2^E * (both bounds) <= 2^14 (|E| <= 100; E = 0 when a bound is not finite).
+ *   lpd_edge_grad_scale_f16   : dx [M][lddx] (point-level gradient of the max), bn, S (lpd_bn_bwd_reduce over dx / zsel),
+ *                               zminmax, W2 -> scale fp32 [2][K]: scale[0][:] = 2^E, scale[1][:] = 2^-E.  work: uint32 [C]
+ *                               scratch.  Two launches (column max of |dx|, then one block for the bounds).
+ * Consumers undo the scale exactly: lpd_edge_bwd_*_f16 take dyscale = scale[1]; dW2 = (2^E dz2e)^T y1 runs on lpd_gemm_f16_tn
+ * and lpd_splitk_reduce with the vector scale[1]; dy1 = dz2e . W2 is linear and runs on lpd_gemm_f16 with fp16 output. */
+int lpd_bn_stats_f16(const void* z, long long rows, int C, int ld, double* partial, int nparts, uint32_t* minmax, void* stream);
+int lpd_edge_materialize_f16(const float* p, int ldp, const float* q, int ldq, const int32_t* idx, int B, int N, int k, int C,
+                             const float* scale, const float* shift, int act, float slope, void* y, void* stream);
+int lpd_edge_sel_dense_f16(const void* z, long long M, int k, int C, const float* gamma, float* zsel, int ldz, uint8_t* arg,
+                           void* stream);
+int lpd_edge_dense_bwd_apply_f16(const void* z, long long M, int k, int C, const float* bn, const float* S, double count,
+                                 int act, float slope, const float* dx, int lddx, const float* zsel, int ldzs,
+                                 const uint8_t* arg, void* dz, const float* gscale, void* stream);
+int lpd_edge_bwd_reduce_f16(const float* p, int ldp, const float* q, int ldq, const int32_t* idx, int B, int N, int k, int C,
+                            const float* bn, int act, float slope, const float* dx, int lddx, const uint8_t* arg,
+                            const void* dy, const float* dyscale, double* partial, int nparts, void* stream);
+int lpd_edge_bwd_apply_f16(const float* p, int ldp, const float* q, int ldq, const int32_t* idx, int B, int N, int k, int C,
+                           const float* bn, int act, float slope, const float* dx, int lddx, const uint8_t* arg,
+                           const void* dy, const float* dyscale, const float* S, double count, float* dp, int lddp,
+                           float* dq, int lddq, void* stream);
+int lpd_edge_grad_scale_f16(const float* dx, int lddx, long long M, int C, const float* bn, const float* S, double count,
+                            int act, float slope, const uint32_t* zminmax, const void* w, int ldw, int K,
+                            uint32_t* work, float* scale, void* stream);
+
 /* backward of the gather-only edges e[(i,m)][:] = f[j(i,m)][:] (get_graph_feature_Origin(cat=False), lpdnet_model.py:116-145;
  * forward = lpd_edge_materialize with q = NULL, scale 1, shift 0, no activation): dp[j] += dy[(i,m)], dp zeroed first. */
 int lpd_edge_scatter_add(const float* dy, const int32_t* idx, int B, int N, int k, int C, float* dp, int lddp, void* stream);

@@ -92,6 +92,14 @@ SIGNATURES = {
     "lpd_edge_bwd_apply": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _vp, _i, _f, _vp, _i, _vp, _vp, _vp, _d,
                                 _vp, _i, _vp, _i, _vp]),
     "lpd_edge_scatter_add": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _vp]),
+    "lpd_bn_stats_f16": (_i, [_vp, _ll, _i, _i, _vp, _i, _vp, _vp]),
+    "lpd_edge_materialize_f16": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _i, _f, _vp, _vp]),
+    "lpd_edge_sel_dense_f16": (_i, [_vp, _ll, _i, _i, _vp, _vp, _i, _vp, _vp]),
+    "lpd_edge_dense_bwd_apply_f16": (_i, [_vp, _ll, _i, _i, _vp, _vp, _d, _i, _f, _vp, _i, _vp, _i, _vp, _vp, _vp, _vp]),
+    "lpd_edge_bwd_reduce_f16": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _vp, _i, _f, _vp, _i, _vp, _vp, _vp, _vp, _i, _vp]),
+    "lpd_edge_bwd_apply_f16": (_i, [_vp, _i, _vp, _i, _vp, _i, _i, _i, _i, _vp, _i, _f, _vp, _i, _vp, _vp, _vp, _vp, _d,
+                                    _vp, _i, _vp, _i, _vp]),
+    "lpd_edge_grad_scale_f16": (_i, [_vp, _i, _ll, _i, _vp, _vp, _d, _i, _f, _vp, _vp, _i, _i, _vp, _vp, _vp]),
     "lpd_netvlad_finish_train": (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "lpd_netvlad_finish_bwd": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp, _vp, _vp]),
     "lpd_softmax64_bwd": (_i, [_vp, _vp, _vp, _ll, _i, _vp]),

@@ -11,7 +11,7 @@ from . import _lib
 from ._lib import (ACT_ADD, ACT_GATE, ACT_LEAKY, ACT_NONE, ACT_RELU, ACT_SIGMOID, A_KM, A_MK, B_KN, B_NK)
 
 __all__ = ["bn_fold", "transpose", "knn", "knn_tc_variant", "pointwise_mlp2", "gemm", "colmax", "edge_gather_ext", "edgeconv_dg",
-           "gemm_tf32", "linear", "set_precision", "get_precision", "netvlad_assign", "softmax64", "netvlad_finish", "splitk_reduce", "quadruplet_loss", "retrieval_topk", "retrieval_tc", "retrieval_search", "recall_count",
+           "gemm_tf32", "linear", "set_precision", "get_precision", "set_train_precision", "get_train_precision", "netvlad_assign", "softmax64", "netvlad_finish", "splitk_reduce", "quadruplet_loss", "retrieval_topk", "retrieval_tc", "retrieval_search", "recall_count",
            "ACT_NONE", "ACT_RELU", "ACT_LEAKY", "ACT_SIGMOID", "ACT_GATE", "A_MK", "A_KM", "B_NK", "B_KN"]
 
 
@@ -856,3 +856,113 @@ def wgrad(dz, lddz, a, lda, rows, Nout, Kin, out=None):
         axpy(out, Kin, res, Kin, Nout, Kin, 1.0)
         return out
     return res
+
+
+# ---- train precision mode -------------------------------------------------------------------------------------------
+#   "default": training runs with the numerics of the precision mode above (fp32 storage of every activation and gradient)
+#   "f16":     the train-mode forward and backward of featnet="lpdnet" keep the four [B*N*k, 128] tensors of the DG2 edge layer in
+#              FP16: y1 (activated DG1 edge rows, rounded to nearest), z2e = y1 . W2^T (lpd_gemm_f16, fp32 accumulate), and their
+#              gradients dz2e and dy1, stored as fp16(2^E * value) with one device-computed power-of-two exponent E per step
+#              (include/lpd_b200.h, "f16 storage of the edge tensors").  Half the bytes of the step's largest tensors and 1.85 GB
+#              less peak memory at 2 x 22 x 4096 points.  Needs get_precision() "tf32" or "f16"; z2e must fit fp16's range
+#              (|z| < 65504), or the loss comes out non-finite.  lpdnetorigin and pointnet training ignore it.
+_train_precision = "default"
+
+
+def set_train_precision(mode: str) -> str:
+    """Select "default" or "f16" storage of the LPD-Net DG2 edge tensors in training; returns the previous mode."""
+    global _train_precision
+    if mode not in ("default", "f16"):
+        raise ValueError("train precision must be 'default' or 'f16'")
+    prev, _train_precision = _train_precision, mode
+    return prev
+
+
+def get_train_precision() -> str:
+    return _train_precision
+
+
+def bn_stats_f16(z, rows, C, ld):
+    """lpd_bn_stats over fp16 z -> (partial, nparts, minmax uint32 keys [2, C])"""
+    lib = _lib.load()
+    _f16(z, "z")
+    nparts = _nparts(rows)
+    part = _partial(nparts, C, z.device)
+    minmax = torch.empty(2, C, device=z.device, dtype=torch.int32)
+    _call(f"lpd_bn_stats_f16[C={C}]", 1, lib.lpd_bn_stats_f16, z.data_ptr(), rows, C, ld, part.data_ptr(), nparts, minmax.data_ptr(),
+          _stream())
+    return part, nparts, minmax
+
+
+def edge_materialize_f16(p, ldp, q, ldq, idx, B, N, k, C, scale, shift, act, slope):
+    lib = _lib.load()
+    y = torch.empty(B * N * k, C, device=p.device, dtype=torch.float16)
+    _call(f"lpd_edge_materialize_f16[C={C}]", 1, lib.lpd_edge_materialize_f16, p.data_ptr(), ldp, _p(q), ldq, idx.data_ptr(), B, N, k, C,
+          scale.data_ptr(), shift.data_ptr(), act, float(slope), y.data_ptr(), _stream())
+    return y
+
+
+def edge_sel_dense_f16(z, M, k, C, gamma):
+    lib = _lib.load()
+    _f16(z, "z")
+    zsel = torch.empty(M, C, device=z.device, dtype=torch.float32)
+    arg = torch.empty(M, C, device=z.device, dtype=torch.uint8)
+    _call(f"lpd_edge_sel_dense_f16[C={C}]", 1, lib.lpd_edge_sel_dense_f16, z.data_ptr(), M, k, C, _p(gamma), zsel.data_ptr(), C,
+          arg.data_ptr(), _stream())
+    return zsel, arg
+
+
+def edge_grad_scale_f16(dx, lddx, M, C, bn, S, count, act, slope, zminmax, w_h):
+    """-> scale fp32 [2, K]: row 0 = 2^E, row 1 = 2^-E, E the exponent of the fp16 edge gradients (lpd_edge_grad_scale_f16);
+    w_h: the layer's fp16 weight [C, K]"""
+    lib = _lib.load()
+    _f16(w_h, "w")
+    K = w_h.shape[1]
+    work = torch.empty(C, device=dx.device, dtype=torch.int32)
+    scale = torch.empty(2, K, device=dx.device, dtype=torch.float32)
+    _call(f"lpd_edge_grad_scale_f16[C={C}]", 2, lib.lpd_edge_grad_scale_f16, dx.data_ptr(), lddx, M, C, bn.data_ptr(), S.data_ptr(),
+          float(count), act, float(slope), zminmax.data_ptr(), w_h.data_ptr(), w_h.stride(0), K, work.data_ptr(), scale.data_ptr(),
+          _stream())
+    return scale
+
+
+def edge_dense_bwd_apply_f16(z, M, k, C, bn, S, count, act, slope, dx, lddx, zsel, arg, gscale):
+    """in place on fp16 z: -> fp16 2^E * dz [M*k, C], gscale[0] = 2^E"""
+    lib = _lib.load()
+    _f16(z, "z")
+    _call(f"lpd_edge_dense_bwd_apply_f16[C={C}]", 1, lib.lpd_edge_dense_bwd_apply_f16, z.data_ptr(), M, k, C, bn.data_ptr(),
+          S.data_ptr(), float(count), act, float(slope), dx.data_ptr(), lddx, zsel.data_ptr(), C, arg.data_ptr(), z.data_ptr(),
+          gscale.data_ptr(), _stream())
+    return z
+
+
+def edge_bwd_f16(p, ldp, q, ldq, idx, B, N, k, C, bn, act, slope, dx, lddx, arg, dy, dyscale, dp, lddp, dq, lddq):
+    """edge_bwd with the dense incoming gradient given as fp16 dy = 2^E * gradient, dyscale[0] = 2^-E"""
+    lib = _lib.load()
+    _f16(dy, "dy")
+    count = B * N * k
+    nparts = SM_COUNT * 8
+    part = _partial(nparts, C, p.device)
+    _call(f"lpd_edge_bwd_reduce_f16[C={C}]", 1, lib.lpd_edge_bwd_reduce_f16, p.data_ptr(), ldp, _p(q), ldq, idx.data_ptr(), B, N, k, C,
+          bn.data_ptr(), act, float(slope), _p(dx), lddx, _p(arg), dy.data_ptr(), dyscale.data_ptr(), part.data_ptr(), nparts, _stream())
+    S = colsum_finalize(part, nparts, 2 * C).view(2, C)
+    _call(f"lpd_edge_bwd_apply_f16[C={C}]", 2, lib.lpd_edge_bwd_apply_f16, p.data_ptr(), ldp, _p(q), ldq, idx.data_ptr(), B, N, k, C,
+          bn.data_ptr(), act, float(slope), _p(dx), lddx, _p(arg), dy.data_ptr(), dyscale.data_ptr(), S.data_ptr(), float(count),
+          dp.data_ptr(), lddp, _p(dq), lddq, _stream())
+    return S
+
+
+def wgrad_f16(dz_h, lddz, a_h, lda, rows, Nout, Kin, scale):
+    """dW[n][k] = scale[k] * sum_r dz_h[r][n] * a_h[r][k] for fp16 operands (the gradient dz_h stored scaled, scale = its inverse
+    scale per output column): lpd_gemm_f16_tn over row slices that are multiples of 64 rows, then the fixed-order
+    lpd_splitk_reduce.  -> fp32 [Nout, Kin]"""
+    bn = 256
+    tiles = ((Nout + 127) // 128) * ((Kin + bn - 1) // bn)
+    want = max(1, min(512, (2 * SM_COUNT + tiles - 1) // tiles, rows // 256 if rows >= 256 else 1))
+    splits = 1
+    while splits * 2 <= want and rows % (splits * 2) == 0 and (rows // (splits * 2)) % 64 == 0:
+        splits *= 2
+    per = rows // splits
+    part = torch.empty(splits, Nout, Kin, device=dz_h.device, dtype=torch.float32)
+    gemm_f16_tn(dz_h, a_h, M=Nout, N=Kin, K=per, lda=lddz, ldb=lda, batch=splits, out=part)
+    return splitk_reduce(part, splits, Nout, Kin, scale=scale)

@@ -281,6 +281,9 @@ class LPDNetTrain:
 
     def fwd(self, x):
         net = self.net
+        self.f16 = ops.get_train_precision() == "f16"
+        if self.f16 and ops.get_precision() == "fp32":
+            raise LpdError('set_train_precision("f16") needs precision "tf32" or "f16": "fp32" stays strict fp32')
         require_cuda(x, "LPDNet")
         B, _, N, D = x.shape
         M, k = B * N, net.k
@@ -310,12 +313,21 @@ class LPDNetTrain:
         self.pyr = torch.empty(M, 512, device=dev, dtype=torch.float32)
         pyr = self.pyr
         ops.affine_act(self.zsel1, M, 128, 128, self.bn1e[0], self.bn1e[1], act, slope, out=pyr, ldo=512)
-        self.y1 = ops.edge_materialize(p1, 256, q1, 256, self.idx_f, B, N, k, 128, self.bn1e[0], self.bn1e[1], act, slope)
         self.wdg2 = w2d(net.convDG2[0].weight)
-        self.z2e = ops.linear(self.y1, self.wdg2, M=M * k, N=128, K=128)
-        part, nparts = ops.bn_stats(self.z2e, M * k, 128, 128)
-        self.bn2e = _bn_finalize(bn_dg2, part, nparts, M * k, 128)
-        self.zsel2, self.arg2 = ops.edge_sel_dense(self.z2e, M, k, 128, bn_dg2.weight.detach())
+        if self.f16:
+            # DG2 edge tensors in fp16 (ops.set_train_precision): y1 rounded to nearest, z2e = y1 . W2^T with fp32 accumulation
+            self.y1 = ops.edge_materialize_f16(p1, 256, q1, 256, self.idx_f, B, N, k, 128, self.bn1e[0], self.bn1e[1], act, slope)
+            self.wdg2_h = ops.to_f16(self.wdg2)
+            self.z2e = ops.gemm_f16(self.y1, self.wdg2_h, M=M * k, N=128, K=128, out_half=True)
+            part, nparts, self.z2e_minmax = ops.bn_stats_f16(self.z2e, M * k, 128, 128)
+            self.bn2e = _bn_finalize(bn_dg2, part, nparts, M * k, 128)
+            self.zsel2, self.arg2 = ops.edge_sel_dense_f16(self.z2e, M, k, 128, bn_dg2.weight.detach())
+        else:
+            self.y1 = ops.edge_materialize(p1, 256, q1, 256, self.idx_f, B, N, k, 128, self.bn1e[0], self.bn1e[1], act, slope)
+            self.z2e = ops.linear(self.y1, self.wdg2, M=M * k, N=128, K=128)
+            part, nparts = ops.bn_stats(self.z2e, M * k, 128, 128)
+            self.bn2e = _bn_finalize(bn_dg2, part, nparts, M * k, 128)
+            self.zsel2, self.arg2 = ops.edge_sel_dense(self.z2e, M, k, 128, bn_dg2.weight.detach())
         ops.affine_act(self.zsel2, M, 128, 128, self.bn2e[0], self.bn2e[1], act, slope, out=pyr[:, 128:], ldo=512)
         # ---- Cartesian graph on the input coordinates: SN1 (decomposed) over x2 -> x3 ---------------------------------
         self.idx_x = ops.knn(xyz, k)
@@ -356,15 +368,26 @@ class LPDNetTrain:
         del dpq3
         # ---- DG2: dense edge layer whose only consumer is the max ----------------------------------------------------
         S2 = ops.bn_bwd_sums(dx2, 512, self.zsel2, 128, M, 128, self.bn2e, act, slope)
-        dz2e = ops.edge_dense_bwd_apply(self.z2e, M, k, 128, self.bn2e, S2, M * k, act, slope, dx2, 512, self.zsel2, self.arg2)
         grads.add(bn_dg2.bias, S2[0])
         grads.add(bn_dg2.weight, S2[1])
-        grads.add(net.convDG2[0].weight, ops.wgrad(dz2e, 128, self.y1, 128, M * k, 128, 128))
-        dy1 = dgrad(dz2e, 128, self.wdg2, M * k, 128, 128, out=self.y1, ldc=128)   # y1 is dead after the wgrad: reuse it
-        # ---- DG1: dense gradient from DG2 + arg-routed gradient of x1 -----------------------------------------------
         dpq1 = torch.empty(M, 256, device=dev, dtype=torch.float32)
-        S1 = ops.edge_bwd(self.pq1, 256, self.pq1[:, 128:], 256, self.idx_f, B, N, k, 128, self.bn1e, act, slope, dpyr, 512,
-                          self.arg1, dy1, dpq1, 256, dpq1[:, 128:], 256)
+        if self.f16:
+            # fp16 gradients stored as 2^E * value: scale = [2^E; 2^-E], E from the bound of include/lpd_b200.h
+            gs = ops.edge_grad_scale_f16(dx2, 512, M, 128, self.bn2e, S2, M * k, act, slope, self.z2e_minmax, self.wdg2_h)
+            dz2e = ops.edge_dense_bwd_apply_f16(self.z2e, M, k, 128, self.bn2e, S2, M * k, act, slope, dx2, 512, self.zsel2, self.arg2, gs[0])
+            grads.add(net.convDG2[0].weight, ops.wgrad_f16(dz2e, 128, self.y1, 128, M * k, 128, 128, gs[1]))
+            w2t_h = ops.to_f16(ops.transpose(self.wdg2.unsqueeze(0))[0])
+            dy1 = ops.gemm_f16(dz2e, w2t_h, M=M * k, N=128, K=128, out=self.y1, ldc=128)      # 2^E * dy1, over the dead y1
+            # ---- DG1: dense gradient from DG2 + arg-routed gradient of x1 -------------------------------------------
+            S1 = ops.edge_bwd_f16(self.pq1, 256, self.pq1[:, 128:], 256, self.idx_f, B, N, k, 128, self.bn1e, act, slope, dpyr, 512,
+                                  self.arg1, dy1, gs[1], dpq1, 256, dpq1[:, 128:], 256)
+        else:
+            dz2e = ops.edge_dense_bwd_apply(self.z2e, M, k, 128, self.bn2e, S2, M * k, act, slope, dx2, 512, self.zsel2, self.arg2)
+            grads.add(net.convDG2[0].weight, ops.wgrad(dz2e, 128, self.y1, 128, M * k, 128, 128))
+            dy1 = dgrad(dz2e, 128, self.wdg2, M * k, 128, 128, out=self.y1, ldc=128)   # y1 is dead after the wgrad: reuse it
+            # ---- DG1: dense gradient from DG2 + arg-routed gradient of x1 -------------------------------------------
+            S1 = ops.edge_bwd(self.pq1, 256, self.pq1[:, 128:], 256, self.idx_f, B, N, k, 128, self.bn1e, act, slope, dpyr, 512,
+                              self.arg1, dy1, dpq1, 256, dpq1[:, 128:], 256)
         grads.add(bn_dg1.bias, S1[0])
         grads.add(bn_dg1.weight, S1[1])
         dwpq1 = ops.wgrad(dpq1, 256, self.h2, 64, M, 256, 64)                      # [256, 64]
